@@ -2,7 +2,7 @@
 """bench.py -- 3D swelling (swelling-3d.py) solve phase on B200: time-to-1e-8, GMRES iteration
 throughput, SpMV HBM roofline.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--mesh-n M]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--mesh-n M] [--dump-outputs DIR]
 
 A "step" is ONE complete `Solver.solve(b, x)` of the assembled three-field system from a zero
 initial guess to relative residual 1e-8 (right-preconditioned GMRES + block `diagonal`
@@ -15,13 +15,16 @@ timed steps (whole job, all ranks; a weaker preconditioner that needs more itera
 D2H inside the timed region).  Iteration throughput, phase profile and the roofline of the dominant kernel
 are measured in a SEPARATE profiled pass after the timed ones.
 
+`--dump-outputs DIR` writes what the last timed step returned to its caller, as float64 .npy files: `x` (the solution,
+`x_rank<r>` per rank when several ranks share the mesh) and `residual_history` (the outer KSP's residual norms).  The
+inputs depend only on the arguments, so two builds run with the same arguments can be compared file by file.
+
 Weak scaling: N GPUs solve the cube with ~N x the DoFs of the 1-GPU mesh, row-partitioned in
 z-slabs (one rank per GPU, NCCL halo exchange + all-reduce).
 
 `--impl reference`: the reference's own stack (petsc4py/dolfin/hypre) is absent from this image
 and unbuildable offline, so the reference arm times the CPU oracle port (numpy/scipy set-up + C/OpenMP solve
-loop restating the same algorithm, oracle/) on the host cores, on the SAME mesh as the GPU arm at that N
-(bounded in the number of solves it repeats, not in the problem).
+loop restating the same algorithm, oracle/) on the host cores, on the SAME mesh as the GPU arm at that N.
 """
 from __future__ import annotations
 
@@ -77,6 +80,23 @@ PHASE_NAMES = {0: "outer_A_apply", 1: "pc_apply", 2: "s_solve", 3: "fp_split0(f)
 RTOL = 1e-8
 METRIC = "3D swelling (swelling-3d.py) solve to rtol 1e-8: DoFs solved per second (n_dofs / time-to-1e-8)"
 UNIT = "DoF/s"
+DUMP_BYTES = 64 * 10 ** 6        # --dump-outputs writes at most this much in all (all ranks together)
+
+
+def dump_outputs(out_dir: str, arrays: dict, budget: int) -> None:
+    """Writes each array as out_dir/<name>.npy in float64, in at most `budget` bytes.  Smaller arrays are written whole first; an
+    array that does not fit its share of what is left is replaced by the entries at a fixed sample of indices (seed 0, ascending
+    order), the same sample in every run with the same arguments."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: np.size(kv[1]))
+    for i, (name, a) in enumerate(items):
+        a = np.ascontiguousarray(a, dtype=np.float64).ravel()
+        cap = (budget // (len(items) - i) - 128) // a.itemsize     # 128 B: the .npy header
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        budget -= os.path.getsize(path)
 
 
 def active_options() -> str:
@@ -256,7 +276,7 @@ def cpu_baseline(mesh_n: int, x_gpu=None):
 
 def run_reference(args):
     """The reference arm: the oracle port's solve of the SAME mesh the GPU arm solves at this N, on all host cores.
-    Each step is one full solve; the number of solves actually repeated is bounded so that the arm ends within minutes."""
+    Each step is one full solve."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -276,34 +296,32 @@ def run_reference(args):
     label = [k for k in runs if k.startswith("C + OpenMP")]
     label = label[0] if label else list(runs)[0]
     run, ncores = runs[label]
-    t0 = time.perf_counter()
-    r = run()                                       # warm-up solve, also the estimate that bounds the repeat count
-    t1 = time.perf_counter() - t0
-    steps_timed = max(1, min(args.steps, int(90.0 / max(t1, 1e-3))))
+    run()                                           # warm-up solve
     for _ in range(max(0, min(args.warmup, 1) - 1)):
         run()
     t0 = time.perf_counter()
     its = 0
-    for _ in range(steps_timed):
+    for _ in range(args.steps):
         r = run()
         its += r.its
-    dt = (time.perf_counter() - t0) / steps_timed
+    dt = (time.perf_counter() - t0) / args.steps
     val = sys_.n / dt
     res = float(np.linalg.norm(sys_.b - sys_.A @ r.x) / np.linalg.norm(sys_.b))
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * dt, "higher_is_better": True, "scaling": "weak",
-            "vs_baseline": None, "dtype": "f64", "data": "synthetic", "steps_timed": steps_timed,
+            "vs_baseline": None, "dtype": "f64", "data": "synthetic", "steps_timed": args.steps,
             "config": {"workload": workload_text(N, sys_.n, sys_.A.nnz, 100, "maxiter", 1), "same_config_as_gpu_arm": same,
                        "gpu_arm_mesh_n": N_arm,
                        "note": "CPU oracle port (numpy set-up + C/OpenMP solve loop), NOT PETSc/hypre; each step = one full "
-                               "solve, %d of the %d requested steps executed (bounded sample)%s" % (
-                                   steps_timed, args.steps, "" if same else "; sample = the 1-GPU mesh (per-GPU share of the "
-                                   "weak-scaled workload): the port's set-up of the N=%d mesh does not fit the time budget" % N_arm)},
-            "time_to_1e-8_s": dt, "its_per_solve": its / steps_timed, "true_rel_residual": res,
+                               "solve%s" % ("" if same else "; sample = the 1-GPU mesh (per-GPU share of the weak-scaled "
+                                            "workload): the port's set-up of the N=%d mesh does not fit the time budget" % N_arm)},
+            "time_to_1e-8_s": dt, "its_per_solve": its / args.steps, "true_rel_residual": res,
             "cpu_baseline": {"value": val, "unit": UNIT, "cores": ncores, "kind": "port",
-                             "sample": "mesh N=%d (%d DoFs), %d full solves, %s; NOT PETSc/hypre" % (N, sys_.n, steps_timed, label)},
+                             "sample": "mesh N=%d (%d DoFs), %d full solves, %s; NOT PETSc/hypre" % (N, sys_.n, args.steps, label)},
             "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"x": r.x, "residual_history": r.history}, DUMP_BYTES)
     print(json.dumps(line))
 
 
@@ -345,7 +363,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--assemble", default="device", choices=["device", "host"],
                     help="device: each rank generates its slab of A, P in HBM (csrc/gen.cu); host: hostfem element assembly + upload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (solution, residual history) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -463,6 +485,7 @@ def main():
     launches = ctx.launch_count() - l0
     reason, rnorm = ksp.reason, ksp.rnorm
     xs = dx.numpy()
+    history = ksp.getConvergenceHistory()
     step_host()
     dt_e, its_e = timed(step_host, args.steps, "e2e")
     clocks = sampler.stop()
@@ -485,6 +508,12 @@ def main():
         dist.all_reduce(sums)
     true_res = float(torch.sqrt(sums[0] / sums[1]))
     ok = reason > 0 and true_res <= 1.01 * RTOL          # the TRUE residual, not the recurrence's estimate
+    if args.dump_outputs:
+        # each rank writes its own rows of x; the residual history is the same on every rank
+        outputs = {"x" if world == 1 else "x_rank%d" % rank: xs}
+        if rank == 0:
+            outputs["residual_history"] = history
+        dump_outputs(args.dump_outputs, outputs, DUMP_BYTES // world)
 
     if rank != 0:
         if world > 1:
