@@ -169,6 +169,12 @@ int poro_pc_inner_solve(poro_pc* pc, const char* name, const double* r_dev, doub
 int poro_pc_inner_result(poro_pc* pc, const char* name, int* its, int* reason, double* rnorm);
 /* AMG hierarchy of a block's inner PC: per level rows and nnz; returns number of levels */
 int poro_pc_amg_info(poro_pc* pc, const char* name, int64_t* rows, int64_t* nnz, int cap, int* nlevels);
+/* sparse LU of a block's inner PC ("s","f","p","fp","diff"; -<prefix>pc_factor_mat_solver_type poro above
+ * -poro_dense_lu_limit rows).  out[0..n) receives, in this order: rows, nnz(L) (strictly lower), nnz(U) (with the
+ * diagonal), explicit zeros stored by supernode amalgamation, supernodes, levels of the supernodal tree, rows of the
+ * largest front, perturbed pivots, device bytes held after set-up, flops of the numeric factorisation, its device time
+ * in microseconds, algorithmic bytes of one application without refinement.  Fails for a block that is not a sparse LU. */
+int poro_pc_factor_info(poro_pc* pc, const char* name, int64_t* out, int n);
 /* live profile of the outer operator product (the dominant SpMV): CUDA events recorded on the
  * launching stream around every y = A x inside poro_ksp_solve.  enable = 1 resets and starts,
  * 0 stops, -1 only reads.  op_bytes = algorithmic bytes of one product

@@ -65,6 +65,7 @@ SIGNATURES = {
     "poro_pc_block_bytes": [vp, C.c_char_p, c_i64p, C.POINTER(C.c_int)],
     "poro_pc_inner_solve": [vp, C.c_char_p, vp, vp],
     "poro_pc_amg_info": [vp, C.c_char_p, c_i64p, c_i64p, C.c_int, C.POINTER(C.c_int)],
+    "poro_pc_factor_info": [vp, C.c_char_p, c_i64p, C.c_int],
     "poro_ksp_mult": [vp, vp, vp],
     "poro_ksp_profile": [vp, C.c_int, c_f64p, c_i64p, c_i64p],
     "poro_profile": [vp, C.c_int, c_f64p, c_i64p, C.c_int],

@@ -462,7 +462,11 @@ static std::unique_ptr<KSP> make_inner(poro_ctx* h, MatOp* op, const std::string
     DistPlan* plan = nullptr;
     if (c.nranks > 1 && (amg_type || pt == "lu") && c.opt_i("-poro_amg_distributed", 1)) plan = op->plan_for_amg();
     const int64_t rows_glob = plan ? plan->offsets.back() : src->nrows;
-    const bool big_lu = pt == "lu" && rows_glob > c.opt_i("-poro_dense_lu_limit", 8192);
+    if (c.nranks > 1 && (pt == "lu" || pt == "cholesky") && c.opt("-" + prefix + "pc_factor_mat_solver_type", "") == "poro")
+        throw Error("-" + prefix + "pc_factor_mat_solver_type poro: the sparse LU factorises a block on one GPU, this block is "
+                    "row-partitioned over " + std::to_string(c.nranks) + " ranks");
+    // with -<prefix>pc_factor_mat_solver_type poro a block above the dense limit is factorised (PCSparseLU, via make_pc)
+    const bool big_lu = pt == "lu" && rows_glob > c.opt_i("-poro_dense_lu_limit", 8192) && !use_sparse_lu(c, pt, prefix, rows_glob);
     if (amg_type || big_lu) {
         // the AMG keeps a pointer to its finest operator: it must live as long as the KSP.  A square block (single rank) or
         // a distributed block with its plan is used in place; otherwise the owned-column part is cut out and kept in owned_op.
@@ -569,7 +573,8 @@ int poro_pc_setup(poro_ctx* h, poro_mat* A, poro_mat* P, poro_mat* P_diff, const
         // which AMG is meaningless, so iterate GMRES on it to 1e-12 with a full Schur factorisation whose sub-blocks
         // are themselves exact (dense) or tightly iterated
         const bool fp_exact_big = fp_pc == "lu" && (nf + np) > c.opt_i("poro_dense_lu_limit", 8192);
-        if (fp_pc != "fieldsplit" && !fp_exact_big) {
+        // ... unless -fp_pc_factor_mat_solver_type poro asks for the sparse LU of the whole block
+        if (fp_pc != "fieldsplit" && (!fp_exact_big || use_sparse_lu(c, fp_pc, "fp_", nf + np))) {
             cc.Mfp_fp = extract_block(h, *Pp, of, of + nf + np, {1, 2});
             cc.ksp_fp = make_inner(h, cc.Mfp_fp.get(), ipc == "lu" ? iksp : "gmres", fp_pc, "fp_", 1, nullptr, 0);
         } else {
@@ -829,6 +834,20 @@ int poro_pc_amg_info(poro_pc* pc, const char* name, int64_t* rows, int64_t* nnz,
     if (!a) { *nlevels = 0; return 0; }
     *nlevels = (int)a->amg.levels.size();
     for (int l = 0; l < *nlevels && l < cap; ++l) { rows[l] = a->amg.op(l).nrows; nnz[l] = a->amg.op(l).nnz; }
+    API_END
+}
+
+int poro_pc_factor_info(poro_pc* pc, const char* name, int64_t* out, int n) {
+    API_BEGIN
+    const std::string nm = name ? name : "";
+    KSP* k = (nm == "s" || nm == "f" || nm == "p" || nm == "fp" || nm == "diff") ? find_ksp(pc, nm) : nullptr;
+    if (!k) throw Error("no such inner solver: " + nm);
+    const PCSparseLU* f = dynamic_cast<const PCSparseLU*>(k->pc);
+    if (!f) throw Error("block '" + nm + "' is not factorised by the sparse LU (its inner PC is " + k->pc->kind() +
+                        "; select it with -" + nm + "_pc_factor_mat_solver_type poro above -poro_dense_lu_limit rows)");
+    const int64_t v[] = {f->n, f->nnz_l, f->nnz_u, f->amalg_zeros, f->nsuper, f->nlevels, f->max_front, f->npert,
+                         f->device_bytes, (int64_t)f->flops, (int64_t)std::llround(f->factor_ms * 1e3), f->apply_bytes};
+    for (int i = 0; i < n; ++i) out[i] = i < (int)(sizeof v / sizeof v[0]) ? v[i] : 0;
     API_END
 }
 

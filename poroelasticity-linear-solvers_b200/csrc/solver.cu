@@ -132,7 +132,8 @@ std::unique_ptr<PC> make_pc(Ctx& c, const std::string& pc_type, const Csr& A, in
     if (pc_type == "none") return std::make_unique<PCNone>(&c, A.nrows);
     if (pc_type == "jacobi") return std::make_unique<PCJacobi>(&c, A);
     bool want_lu = pc_type == "lu" || pc_type == "cholesky";
-    if (want_lu && !plan && A.nrows <= c.opt_i("-poro_dense_lu_limit", 8192)) return std::make_unique<PCDense>(&c, A);
+    if (!plan && use_sparse_lu(c, pc_type, prefix, A.nrows)) return std::make_unique<PCSparseLU>(&c, A, prefix);
+    if (want_lu && !plan && A.nrows <=c.opt_i("-poro_dense_lu_limit", 8192)) return std::make_unique<PCDense>(&c, A);
     const bool cheb_only = pc_type == "chebyshev";      // Chebyshev(degree) on D^-1 A = a one-level hierarchy
     if (want_lu || cheb_only || pc_type == "hypre" || pc_type == "amg" || pc_type == "gamg" || pc_type == "ml") {
         auto pc = std::make_unique<PCAmg>();

@@ -84,6 +84,37 @@ struct PCDense : PC {   // exact block solve: explicit inverse (stands in for MU
     const char* kind() const override { return "lu(dense)"; }
 };
 
+// one supernode of PCSparseLU: pivot rows [first, first + k) of the permuted block, a front of m rows
+struct SluNode {
+    int first, k, m, child_begin, child_end;
+    int64_t rows, upd, front, fac;   // offsets: row list, update rows (relmap / update vectors), set-up front, stored factor
+};
+
+// exact block solve by a multifrontal sparse LU (sparse_lu.cu, symbolic analysis in lu_symbolic.h): selected for `lu` /
+// `cholesky` blocks above -poro_dense_lu_limit rows by -<prefix>pc_factor_mat_solver_type poro (use_sparse_lu)
+struct PCSparseLU : PC {
+    Ctx* ctx; int n;
+    DBuf<SluNode> sn;
+    DBuf<int> relmap, child, row_idx, level_sn, perm;
+    std::vector<int> level_ptr;
+    int nlevels = 0;
+    size_t smem = 0;                 // dynamic shared memory of the solve kernels: the largest front
+    DBuf<double> fac, xw, wbuf;      // factors; permuted work vector; per-supernode update vectors
+    // perturbed pivots: one step of iterative refinement with the block (y += LU^-1 (x - B y)), like PCDense
+    Csr A; DBuf<double> r, d;
+    // factor_info
+    int64_t nnz_l = 0, nnz_u = 0, amalg_zeros = 0, npert = 0, device_bytes = 0, apply_bytes = 0;
+    int nsuper = 0, max_front = 0;
+    double flops = 0.0, factor_ms = 0.0;
+    PCSparseLU(Ctx* c, const Csr& A, const std::string& prefix);
+    void apply(const double* x, double* y) override;
+    const char* kind() const override { return "lu(sparse)"; }
+  private:
+    void solve(const double* b, double* x);
+};
+// the block of `prefix` (pc type `pc_type`, `rows` rows) is factorised by PCSparseLU
+bool use_sparse_lu(const Ctx& c, const std::string& pc_type, const std::string& prefix, int64_t rows);
+
 struct PCAmg : PC {
     Amg amg;
     void apply(const double* x, double* y) override { amg.apply(x, y); }

@@ -92,6 +92,16 @@ class PreconditionerCC(object):
         _capi.check(self.ctx.lib.poro_pc_amg_info(self.h, name.encode(), rows, nnz, 32, C.byref(nl)))
         return [(rows[i], nnz[i]) for i in range(nl.value)]
 
+    FACTOR_INFO_KEYS = ("rows", "nnz_l", "nnz_u", "amalgamation_zeros", "supernodes", "levels", "max_front",
+                        "perturbed_pivots", "device_bytes", "factor_flops", "factor_us", "apply_bytes")
+
+    def factor_info(self, name):
+        """Sparse LU of a block's inner PC ("s","f","p","fp","diff") as a dict (keys: FACTOR_INFO_KEYS, see
+        poro_pc_factor_info in include/poro.h); raises for a block that is not factorised by the sparse LU."""
+        out = (C.c_int64 * len(self.FACTOR_INFO_KEYS))()
+        _capi.check(self.ctx.lib.poro_pc_factor_info(self.h, name.encode(), out, len(out)))
+        return dict(zip(self.FACTOR_INFO_KEYS, (int(v) for v in out)))
+
     def inner_solve(self, name, r, z):
         _capi.check(self.ctx.lib.poro_pc_inner_solve(self.h, name.encode(), _capi._ptr(_tensor(r)), _capi._ptr(_tensor(z))))
 
