@@ -157,9 +157,15 @@ int poro_aar_destroy(poro_aar* aar);
 /* ---- micro-benchmark / introspection entry points ----------------------------------------- */
 /* block names: "A" (whole permuted operator), "ss","sf","sp","fs","ff","fp","ps","pf","pp" of P */
 int poro_pc_block_info(poro_pc* pc, const char* name, int64_t* nrows, int64_t* ncols, int64_t* nnz);
-/* algorithmic bytes of one product y = B x with a block in the format it is launched in (0 CSR, 1 BSR, 2 diagonal BSR):
- * 12 nnz + 4 (nrows+1) + 8 nrows + 8 ncols, or (8 BS^2 + 4) nnzb + 4 (nbrows+1) + 8 nrows + 8 ncols */
+/* algorithmic bytes of one product y = B x with a block in the format it is launched in (0 CSR, 1 BSR, 2 diagonal BSR,
+ * 4 stencil): 12 nnz + 4 (nrows+1) + 8 nrows + 8 ncols, or (8 BS^2 + 4) nnzb + 4 (nbrows+1) + 8 nrows + 8 ncols, or for a
+ * generated block applied from its class tables 8 ncols + table bytes + Dirichlet flags (1 B per row) + 8 nrows */
 int poro_pc_block_bytes(poro_pc* pc, const char* name, int64_t* bytes, int* format);
+/* one product with a block in the path its solvers use, on device vectors (tests of the product kernels):
+ * mode 0 y = B x, 1 y = z - B x, 2 y = z + B x, 3 Chebyshev step (x = d_old; r -= B x; d_new = c1 x + c2 dinv.*r; xv += d_new),
+ * 4 y = B x and *dot = x . y (dot: one device double).  Unused pointers may be null. */
+int poro_pc_block_mult(poro_pc* pc, const char* name, int mode, const double* x, double* y, const double* z, double* r, double* d_new,
+                       double* xv, const double* dinv, double c1, double c2, double* dot);
 /* copy a block to host CSR arrays sized from poro_pc_block_info (tests: createSubMatrix parity) */
 int poro_pc_block_copy(poro_pc* pc, const char* name, int64_t* rowptr, int32_t* col, double* val);
 /* one application of the inner solver of a block: "s","f","p","fp","diff" (z = K \ r) */

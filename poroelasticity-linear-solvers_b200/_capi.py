@@ -63,6 +63,7 @@ SIGNATURES = {
     "poro_pc_block_info": [vp, C.c_char_p, c_i64p, c_i64p, c_i64p],
     "poro_pc_block_copy": [vp, C.c_char_p, vp, vp, vp],
     "poro_pc_block_bytes": [vp, C.c_char_p, c_i64p, C.POINTER(C.c_int)],
+    "poro_pc_block_mult": [vp, C.c_char_p, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_double, C.c_double, vp],
     "poro_pc_inner_solve": [vp, C.c_char_p, vp, vp],
     "poro_pc_amg_info": [vp, C.c_char_p, c_i64p, c_i64p, C.c_int, C.POINTER(C.c_int)],
     "poro_pc_factor_info": [vp, C.c_char_p, c_i64p, C.c_int],

@@ -393,6 +393,14 @@ int poro_fields_set_coords(poro_ctx* h, int dim, const double* coords_s, const d
 // ---------------------------------------------------------------------------------------------
 // block extraction helpers
 // ---------------------------------------------------------------------------------------------
+// the fields of the solver are the generator's fields in the generator's order, and nothing lives in a halo
+static bool stencil_layout_matches(const Fields& fl, const StencilOp& s) {
+    if (!fl.identity) return false;
+    for (int t = 0; t < 3; ++t)
+        if (fl.nh[t] || fl.off[t] != s.d->row0[t] || fl.n[t] != s.d->row0[t + 1] - s.d->row0[t]) return false;
+    return true;
+}
+
 // columns: list of (field) pieces in order; rows: contiguous permuted range [r0, r1)
 static std::unique_ptr<MatOp> extract_block(poro_ctx* h, const Csr& Mp, int64_t r0, int64_t r1, std::vector<int> col_fields) {
     Ctx& c = h->c;
@@ -421,13 +429,27 @@ static std::unique_ptr<MatOp> extract_block(poro_ctx* h, const Csr& Mp, int64_t 
     PORO_CUDA(cudaMemcpy(d_r.p, rmap.data(), rmap.size() * 4, cudaMemcpyHostToDevice));
     PORO_CUDA(cudaMemcpy(d_c.p, cmap.data(), cmap.size() * 4, cudaMemcpyHostToDevice));
     csr_extract(c, Mp, d_r.p, d_c.p, (int)(r1 - r0), (int)pos, op->M);
+    // a generated matrix cut along whole fields (one row field x one column field) keeps its tables: the block's products
+    // run from them (stencil.cu).  Partial ranges, several column fields and permuted matrices stay assembled.
+    if (Mp.stencil && Mp.stencil->fr < 0 && c.nranks == 1 && col_fields.size() == 1 && stencil_layout_matches(fl, *Mp.stencil)) {
+        for (int fr = 0; fr < 3; ++fr)
+            if (fl.n[fr] > 0 && r0 == fl.off[fr] && r1 == fl.off[fr] + fl.n[fr]) {
+                op->M.stencil = std::make_shared<StencilOp>(StencilOp{Mp.stencil->d, fr, col_fields[0]});
+                break;
+            }
+    }
     return op;
 }
 
 // square local part (owned columns only) of a block operator: what the inner PCs are built on
 static void local_square(Ctx& c, const MatOp& op, Csr& out) {
     const Csr& M = op.mat();
-    if (M.ncols == M.nrows) { csr_copy(c, M, out); PORO_CUDA(cudaStreamSynchronize(c.stream)); return; }
+    if (M.ncols == M.nrows) {
+        csr_copy(c, M, out);
+        out.stencil = M.stencil;        // the same operator
+        PORO_CUDA(cudaStreamSynchronize(c.stream));
+        return;
+    }
     std::vector<int> rmap((size_t)M.nrows), cmap((size_t)M.ncols, -1);
     for (int i = 0; i < M.nrows; ++i) { rmap[i] = i; cmap[i] = i; }
     DBuf<int> d_r(rmap.size()), d_c(cmap.size());
@@ -764,12 +786,18 @@ int poro_pc_block_info(poro_pc* pc, const char* name, int64_t* nrows, int64_t* n
     API_END
 }
 
-// algorithmic bytes of ONE plain product y = B x with a block in the format it is launched in (0 CSR, 1 BSR, 2 diagonal BSR)
+// algorithmic bytes of ONE plain product y = B x with a block in the format it is launched in (0 CSR, 1 BSR, 2 diagonal BSR,
+// 4 stencil: generated block applied from its class tables)
 int poro_pc_block_bytes(poro_pc* pc, const char* name, int64_t* bytes, int* format) {
     API_BEGIN
     MatOp* m = find_block(pc, name);
     if (!m) throw Error(std::string("no such block: ") + name);
     const Csr& B = m->mat();
+    if (B.stencil && B.stencil->fr >= 0) {
+        *bytes = stencil_bytes(*B.stencil);
+        *format = 4;
+        return 0;
+    }
     csr_ensure_bsr(pc->ctx->c, B);
     if (B.bsr_state == 1) {
         const Bsr& b = *B.bsr;
@@ -780,6 +808,22 @@ int poro_pc_block_bytes(poro_pc* pc, const char* name, int64_t* bytes, int* form
         *bytes = 12 * B.nnz + 4 * ((int64_t)B.nrows + 1) + 8 * (int64_t)B.nrows + 8 * (int64_t)B.ncols;
         *format = 0;
     }
+    API_END
+}
+
+int poro_pc_block_mult(poro_pc* pc, const char* name, int mode, const double* x, double* y, const double* z, double* r, double* d_new,
+                       double* xv, const double* dinv, double c1, double c2, double* dot) {
+    API_BEGIN
+    MatOp* m = find_block(pc, name);
+    if (!m) throw Error(std::string("no such block: ") + name);
+    Ctx& c = pc->ctx->c;
+    const Csr& B = m->mat();
+    PORO_REQUIRE(mode >= 0 && mode <= 4, "mode in 0..4");
+    PORO_REQUIRE(mode <= 2 || B.nrows == B.ncols, "Chebyshev / dot modes need a square block");
+    if (mode <= 2) m->apply(x, y, (SpmvMode)mode, z);
+    else if (mode == 3) spmv_cheb_step(c, B, x, x, d_new, r, xv, dinv, c1, c2);
+    else spmv_dot(c, B, x, y, dot);
+    PORO_CUDA(cudaStreamSynchronize(c.stream));
     API_END
 }
 
@@ -868,6 +912,12 @@ static std::unique_ptr<MatOp> make_outer_op(poro_ctx* h, poro_mat* A) {
     for (int t = 0; t < 3; ++t)
         if (fl.nh[t] || c.nranks > 1) op->pieces.push_back({&fl.halo[t], fl.off[t], fl.n_owned + fl.hoff[t]});
     if (!op->ref) csr_choose_lanes(op->M);
+    // generated matrix on one rank: one stencil launch per row field, each summing the row field's tables (stencil.cu)
+    if (op->ref && A->raw.stencil && A->raw.stencil->fr < 0 && c.nranks == 1 && stencil_layout_matches(fl, *A->raw.stencil)) {
+        for (int fr = 0; fr < 3; ++fr)
+            if (fl.n[fr] > 0) op->stencil_rows.push_back(std::make_shared<StencilOp>(StencilOp{A->raw.stencil->d, fr, -1}));
+        return op;
+    }
     // node-blocked s and f diagonal blocks (owned columns) -> BSR parts; everything else stays in one CSR remainder
     const int bd = fl.block_dim;
     if (bd > 1 && fl.n[0] % bd == 0 && fl.n[1] % bd == 0 && c.opt_i("-poro_use_bsr", 1)) {
@@ -1000,9 +1050,11 @@ int poro_ksp_profile(poro_ksp* k, int enable, double* op_ms, int64_t* op_calls, 
     if (op_ms) *op_ms = s.op_ms;
     if (op_calls) *op_calls = s.op_calls;
     if (op_bytes) {
-        // algorithmic bytes of the formats actually launched: CSR remainder + BSR diagonal parts
+        // algorithmic bytes of the formats actually launched: CSR remainder + BSR diagonal parts, or the stencil launches
         const Csr& A = k->A->mat();
-        int64_t bytes = 12 * A.nnz + 4 * ((int64_t)A.nrows + 1) + 8 * (int64_t)A.nrows + 8 * (int64_t)A.ncols;
+        int64_t bytes = 0;
+        for (auto& s : k->A->stencil_rows) bytes += stencil_bytes(*s);
+        if (k->A->stencil_rows.empty()) bytes += 12 * A.nnz + 4 * ((int64_t)A.nrows + 1) + 8 * (int64_t)A.nrows + 8 * (int64_t)A.ncols;
         for (auto& p : k->A->parts) {
             const Csr& B = p->B;
             if (B.bsr_state == 1) {
@@ -1017,11 +1069,18 @@ int poro_ksp_profile(poro_ksp* k, int enable, double* op_ms, int64_t* op_calls, 
     API_END
 }
 
-// algorithmic bytes of each launch of the outer operator: [CSR remainder, part 0, part 1, ...]; returns count in *n
+// algorithmic bytes of each launch of the outer operator: [CSR remainder, part 0, part 1, ...], or one stencil launch per
+// row field (format 4) for a generated matrix; returns count in *n
 int poro_ksp_parts_info(poro_ksp* k, int64_t* bytes, int* is_bsr, int cap, int* n) {
     API_BEGIN
     std::vector<int64_t> b;
     std::vector<int> f;
+    if (!k->A->stencil_rows.empty()) {
+        for (auto& s : k->A->stencil_rows) { b.push_back(stencil_bytes(*s)); f.push_back(4); }
+        *n = (int)b.size();
+        for (int i = 0; i < *n && i < cap; ++i) { bytes[i] = b[i]; is_bsr[i] = f[i]; }
+        return 0;
+    }
     const Csr& A = k->A->mat();
     b.push_back(12 * A.nnz + 4 * ((int64_t)A.nrows + 1) + 8 * (int64_t)A.nrows + 8 * (int64_t)A.ncols);
     f.push_back(0);

@@ -231,6 +231,8 @@ struct Bsr {
     DBuf<double> t_val, t_m;                 // values (32-interleaved per chunk); one coupling scalar per block (fused)
 };
 
+struct StencilOp;   // stencil.cuh
+
 // ---- sparse matrix (device CSR, local rows) ---------------------------------------------------
 struct Csr {
     int nrows = 0, ncols = 0;
@@ -247,6 +249,8 @@ struct Csr {
     mutable bool fp32_hint = false;             // store the BSR values in fp32 (preconditioner matrices only, opt-in)
     mutable int bsr_state = -1;                 // -1 not tried, 0 rejected (fill-in / shape), 1 in use
     mutable std::shared_ptr<Bsr> bsr;
+    // generated structured-mesh matrix (stencil.cuh): products run from the class tables instead of the CSR (single rank)
+    std::shared_ptr<StencilOp> stencil;
     double avg_row() const { return nrows ? (double)nnz / nrows : 0.0; }
 };
 

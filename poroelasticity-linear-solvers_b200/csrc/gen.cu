@@ -13,6 +13,7 @@
 //                 the row and compact the non-zeros with a ballot, so stores are contiguous
 #include "common.cuh"
 #include "gen_stencil.cuh"
+#include "stencil.cuh"
 #include "../../include/poro.h"
 #include <cub/cub.cuh>
 
@@ -147,22 +148,49 @@ int poro_gen_matrix(poro_ctx* h, int dim, int N, const poro_gen_table* tables, c
         const int64_t nrows = g.row0[3];
         PORO_REQUIRE(nrows < 2147483647LL && ncols < 2147483647LL, "local system too large for 32-bit indices");
         for (int f = 0; f < 3; ++f) PORO_REQUIRE(g.off_owned[f] == g.row0[f], "owned column offsets must equal the row offsets (field-major)");
-        // tables to the device
+        // tables to the device; entries whose block is all zero are dropped (they add nothing to the CSR and only cost the
+        // stencil kernel work), and tables of diagonal blocks are marked for the stencil kernel
         GenTables T{};
         std::vector<DBuf<int32_t>> d_cls(9);
         std::vector<DBuf<int64_t>> d_off(9);
         std::vector<DBuf<double>> d_val(9);
+        int diag_only[9] = {0};
+        int64_t table_bytes[9] = {0};
         for (int b = 0; b < 9; ++b) {
             const poro_gen_table& s = tables[b];
             T.present[b] = s.cls_ptr != nullptr && s.ncls > 0 && s.cls_ptr[s.ncls] > 0;
             if (!T.present[b]) continue;
             const int fr = b / 3, fc = b % 3;
             PORO_REQUIRE(s.kr == g.kind[fr] && s.kc == g.kind[fc] && s.br == g.bdim[fr] && s.bc == g.bdim[fc], "block table does not match its field pair");
-            const int nent = s.cls_ptr[s.ncls];
-            d_cls[b].alloc((size_t)s.ncls + 1); d_off[b].alloc((size_t)nent); d_val[b].alloc((size_t)nent * s.br * s.bc);
-            PORO_CUDA(cudaMemcpyAsync(d_cls[b].p, s.cls_ptr, ((size_t)s.ncls + 1) * 4, cudaMemcpyHostToDevice, c.stream));
-            PORO_CUDA(cudaMemcpyAsync(d_off[b].p, s.off, (size_t)nent * 8, cudaMemcpyHostToDevice, c.stream));
-            PORO_CUDA(cudaMemcpyAsync(d_val[b].p, s.vals, (size_t)nent * s.br * s.bc * 8, cudaMemcpyHostToDevice, c.stream));
+            const int bsz = s.br * s.bc;
+            std::vector<int32_t> cp(1, 0);
+            std::vector<int64_t> of;
+            std::vector<double> va;
+            bool diag = s.br == s.bc;
+            for (int k = 0; k < s.ncls; ++k) {
+                for (int p = s.cls_ptr[k]; p < s.cls_ptr[k + 1]; ++p) {
+                    const double* v = s.vals + (int64_t)p * bsz;
+                    bool nz = false;
+                    for (int q = 0; q < bsz; ++q) {
+                        nz = nz || v[q] != 0.0;
+                        if (v[q] != 0.0 && q / s.bc != q % s.bc) diag = false;
+                    }
+                    if (!nz) continue;
+                    of.push_back(s.off[p]);
+                    va.insert(va.end(), v, v + bsz);
+                }
+                cp.push_back((int32_t)of.size());
+            }
+            diag_only[b] = diag;
+            const int nent = (int)of.size();
+            d_cls[b].alloc(cp.size()); d_off[b].alloc((size_t)nent); d_val[b].alloc(va.size());
+            PORO_CUDA(cudaMemcpyAsync(d_cls[b].p, cp.data(), cp.size() * 4, cudaMemcpyHostToDevice, c.stream));
+            if (nent) {
+                PORO_CUDA(cudaMemcpyAsync(d_off[b].p, of.data(), of.size() * 8, cudaMemcpyHostToDevice, c.stream));
+                PORO_CUDA(cudaMemcpyAsync(d_val[b].p, va.data(), va.size() * 8, cudaMemcpyHostToDevice, c.stream));
+            }
+            PORO_CUDA(cudaStreamSynchronize(c.stream));     // the host vectors go out of scope
+            table_bytes[b] = (int64_t)cp.size() * 4 + (int64_t)nent * 8 + (int64_t)va.size() * 8;
             T.t[b] = porogen::BlockTable{dim, N, s.kr, s.kc, s.br, s.bc, s.diag_block, d_cls[b].p, d_off[b].p, d_val[b].p};
         }
         DBuf<uint8_t> d_bc;
@@ -204,6 +232,38 @@ int poro_gen_matrix(poro_ctx* h, int dim, int N, const poro_gen_table* tables, c
         PORO_CUDA(cudaStreamSynchronize(c.stream));
         PORO_REQUIRE(herr == 0, "generator: a stencil entry falls outside the owned and ghost node ranges of the layout");
         csr_choose_lanes(A);
+        // single rank, whole lattices owned: keep the tables next to the CSR so that products run from them (stencil.cu).
+        // Row-partitioned slabs order their ghost columns differently from the field blocks extracted later: assembled only.
+        bool whole = c.nranks == 1;
+        for (int k = 0; k < 2; ++k)
+            whole = whole && g.o0[k] == 0 && g.o1[k] == porogen::lattice_nodes(k + 1, N, dim) && g.gl0[k] == g.gl1[k] && g.gu0[k] == g.gu1[k];
+        whole = whole && ncols == nrows;
+        if (whole && bc_flags_host) {
+            // the kernel reads the Dirichlet flags of boundary nodes only
+            for (int64_t r = 0; r < nrows && whole; ++r) {
+                if (!bc_flags_host[r]) continue;
+                int f = r < g.row0[1] ? 0 : (r < g.row0[2] ? 1 : 2);
+                int64_t node = (r - g.row0[f]) / g.bdim[f];
+                const int L = porogen::lattice_extent(g.kind[f], N);
+                bool bnd = false;
+                for (int m = 0; m < dim; ++m, node /= L) bnd = bnd || node % L == 0 || node % L == L - 1;
+                whole = bnd;
+            }
+        }
+        if (whole) {
+            auto d = std::make_shared<StencilData>();
+            d->dim = dim; d->N = N;
+            for (int b = 0; b < 9; ++b) {
+                d->t[b] = T.t[b]; d->present[b] = T.present[b]; d->diag_only[b] = diag_only[b]; d->table_bytes[b] = table_bytes[b];
+                d->cls[b] = std::move(d_cls[b]); d->off[b] = std::move(d_off[b]); d->val[b] = std::move(d_val[b]);
+            }
+            d->bc = std::move(d_bc);
+            for (int f = 0; f < 4; ++f) d->row0[f] = g.row0[f];
+            for (int f = 0; f < 3; ++f) { d->bdim[f] = g.bdim[f]; d->kind[f] = g.kind[f]; }
+            stencil_build_warps(c, *d);
+            A.stencil = std::make_shared<StencilOp>();
+            A.stencil->d = std::move(d);
+        }
         *out = poro_mat_adopt(h, std::move(A));
         return 0;
     } catch (const std::exception& e) {

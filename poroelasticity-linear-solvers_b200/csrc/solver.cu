@@ -53,6 +53,15 @@ void MatOp::apply(const double* x, double* y, SpmvMode mode, const double* z) {
     const Csr& A = mat();
     // the halo exchange is collective: every rank runs it, also one whose local block is empty
     const double* xe = extended(x);
+    if (!stencil_rows.empty()) {
+        int ip = 0;
+        for (auto& s : stencil_rows) {
+            ProfScope ps(*ctx, 33 + ip++);
+            const int64_t o = s->d->row0[s->fr];
+            stencil_spmv(*ctx, *s, xe, y + o, mode, z ? z + o : nullptr);
+        }
+        return;
+    }
     const bool prof = !parts.empty();
     if (A.nnz == 0) {                               // structurally empty block (or everything lives in `parts`)
         if (mode == SPMV_SET) vec_set(*ctx, y, 0.0, A.nrows);

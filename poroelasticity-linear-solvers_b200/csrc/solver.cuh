@@ -4,6 +4,7 @@
 #include "common.cuh"
 #include "dist.cuh"
 #include "distamg.cuh"
+#include "stencil.cuh"
 
 namespace poro {
 
@@ -48,6 +49,8 @@ struct MatOp : LinOp {
     // x2_off >= 0: a mass coupling rides along B (bsr_tma.cu, FUSE): y[row_off..] += B x[col_off..] + C x[x2_off..]
     struct DiagPart { Csr B; int64_t row_off, col_off; int64_t x2_off = -1; };
     std::vector<std::unique_ptr<DiagPart>> parts;
+    // outer operator of a generated matrix on one rank: one stencil launch per row field (stencil.cu) instead of M / parts
+    std::vector<std::shared_ptr<StencilOp>> stencil_rows;
     DBuf<double> xext;
     int64_t rows() const override { return mat().nrows; }
     void apply(const double* x, double* y, SpmvMode mode = SPMV_SET, const double* z = nullptr) override;

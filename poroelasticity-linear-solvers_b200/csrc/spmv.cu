@@ -16,6 +16,7 @@
 // HBM-bound: algorithmic bytes = 12 nnz + 4 (nrows+1) + 8 nrows + 8 ncols.
 #include "common.cuh"
 #include "spmv_epilogue.cuh"
+#include "stencil.cuh"
 #include <algorithm>
 
 namespace poro {
@@ -199,6 +200,8 @@ static void try_bsr(Ctx& c, const Csr& A) {
 template <int MODE>
 static int launch_spmv(Ctx& c, const Csr& A, const double* x, double* y, const Epilogue& ep, double* dot_partial) {
     if (A.nrows == 0) return 0;
+    // a generated block along whole fields: apply its class tables (stencil.cu) instead of streaming the assembled matrix
+    if (A.stencil && A.stencil->fr >= 0) return stencil_launch<MODE>(c, *A.stencil, x, y, ep, dot_partial);
     if (A.block_hint > 1 && A.bsr_state < 0) try_bsr(c, A);
     if (A.bsr_state == 1) return bsr_launch<MODE>(c, *A.bsr, x, y, ep, dot_partial);
     if (A.nblk < 0) build_row_blocks(c, A);
@@ -269,9 +272,11 @@ __global__ void k_sum_to(const double* __restrict__ partial, int n, double* __re
 void spmv_dot(Ctx& c, const Csr& A, const double* p, double* w, double* d_dot) {
     Epilogue ep{};
     ep.mode = 4;
-    if (A.nblk < 0) build_row_blocks(c, A);
+    const bool st = A.stencil && A.stencil->fr >= 0;
+    if (!st && A.nblk < 0) build_row_blocks(c, A);
     const int L = A.lanes ? A.lanes : 32;
-    const int64_t grid = A.nblk > 0 ? A.nblk : ceil_div((int64_t)A.nrows * L, kSpmvBlock);   // upper bound for BSR too
+    const int64_t grid = st ? stencil_grid(*A.stencil)
+                            : A.nblk > 0 ? A.nblk : ceil_div((int64_t)A.nrows * L, kSpmvBlock);   // upper bound for BSR too
     if (grid <= Ctx::kScal) {
         int g = launch_spmv<4>(c, A, p, w, ep, c.d_scal);
         k_sum_to<<<1, 256, 0, c.stream>>>(c.d_scal, g, d_dot);

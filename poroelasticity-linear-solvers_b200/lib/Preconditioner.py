@@ -74,7 +74,7 @@ class PreconditionerCC(object):
         return r.value, c.value, z.value
 
     def block_bytes(self, name):
-        """(algorithmic bytes of one product with the block, format 0 CSR / 1 BSR / 2 diagonal BSR)."""
+        """(algorithmic bytes of one product with the block, format 0 CSR / 1 BSR / 2 diagonal BSR / 4 stencil)."""
         b, f = C.c_int64(), C.c_int()
         _capi.check(self.ctx.lib.poro_pc_block_bytes(self.h, name.encode(), C.byref(b), C.byref(f)))
         return b.value, f.value

@@ -53,7 +53,7 @@ class _KSP:
         return ms.value, calls.value, nbytes.value
 
     def parts_info(self):
-        """[(algorithmic bytes, format)] of each launch of the outer operator (format 0 CSR, 1 BSR, 2 diagonal BSR)."""
+        """[(algorithmic bytes, format)] of each launch of the outer operator (format 0 CSR, 1 BSR, 2 diagonal BSR, 3 fused BSR, 4 stencil)."""
         b, f, n = (C.c_int64 * 16)(), (C.c_int * 16)(), C.c_int()
         _capi.check(self.ctx.lib.poro_ksp_parts_info(self.h, b, f, 16, C.byref(n)))
         return [(b[i], f[i]) for i in range(n.value)]
