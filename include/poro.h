@@ -67,6 +67,20 @@ int poro_mat_mult(poro_mat* m, const double* x_dev, double* y_dev);
  * `mult` + `aypx(-1)` pairs, lib/Preconditioner.py:180-199): 0 y = A x, 1 y = z - A x, 2 y = z + A x, 3 Chebyshev step,
  * 4 w = A p with p.w.  Returns the device time per launch (CUDA events on the library's stream). */
 int poro_mat_bench(poro_mat* m, int mode, int reps, double* ms_per_launch);
+/* tests of the product kernels on a raw matrix (single rank).  `-poro_mat_block_hint BS` at creation makes the first product
+ * try BSR, `-poro_mat_fp32_values 1` stores those BSR values in fp32; the `-poro_bsr_*` options are read at that conversion.
+ * poro_mat_mult_mode: one product in the epilogue modes of poro_pc_block_mult.
+ * poro_mat_kernel_info: what the next product launches (converting first, as a product would).  out[0..n) receives:
+ * format (0 CSR stream, 1 BSR, 2 diagonal BSR, 4 stencil, 5 vector-CSR fallback), lanes per row or block row (G of the
+ * stream kernels, L of the fallback), block size, PREF, cooperative gathers, fp32 values, TMA layout, TMA config (-1
+ * none), fused coupling, chunks (row blocks of the CSR stream, chunks of the BSR kernels), L2 prefetch.
+ * poro_mat_mult_fused: modes 0..2 of y = A x + C x2; the first call tries to let C ride along A's BSR (*fused = 1),
+ * otherwise A and C are applied one after the other (*fused = 0). */
+int poro_mat_mult_mode(poro_mat* m, int mode, const double* x, double* y, const double* z, double* r, double* d_new, double* xv,
+                       const double* dinv, double c1, double c2, double* dot);
+int poro_mat_kernel_info(poro_mat* m, int64_t* out, int n);
+int poro_mat_mult_fused(poro_mat* a, poro_mat* c, int mode, const double* x, const double* x2, double* y, const double* z,
+                        int* fused);
 
 int poro_mat_copy(poro_mat* m, int64_t* rowptr, int32_t* col, double* val);
 

@@ -37,6 +37,9 @@ SIGNATURES = {
     "poro_mat_mult": [vp, vp, vp],
     "poro_mat_bench": [vp, C.c_int, C.c_int, c_f64p],
     "poro_mat_copy": [vp, vp, vp, vp],
+    "poro_mat_mult_mode": [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_double, C.c_double, vp],
+    "poro_mat_kernel_info": [vp, c_i64p, C.c_int],
+    "poro_mat_mult_fused": [vp, vp, C.c_int, vp, vp, vp, vp, C.POINTER(C.c_int)],
     "poro_gen_matrix": [vp, C.c_int, C.c_int, vp, vp, vp, C.POINTER(vp)],
     "poro_halo_set": [vp, C.c_int64, C.c_int, vp, vp, vp, vp],
     "poro_fields_set": [vp, vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int, C.c_int],

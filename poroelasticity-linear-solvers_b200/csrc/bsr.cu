@@ -317,7 +317,8 @@ bool bsr_from_csr(Ctx& c, const Csr& A, int BS, Bsr& out, double max_fill) {
                 int lo = b0, hi = b1;
                 while (lo < hi) { int mid = (lo + hi) >> 1; if (bcc[mid] < J) lo = mid + 1; else hi = mid; }
                 const size_t p = (size_t)lo;
-                bv[((p >> 5) * NE + (size_t)(diag ? ri : ri * BS + rj)) * 32 + (p & 31)] = av[k];
+                // summed: an uploaded CSR may repeat an entry, and the CSR kernels add every copy
+                bv[((p >> 5) * NE + (size_t)(diag ? ri : ri * BS + rj)) * 32 + (p & 31)] += av[k];
             }
         });
     }
@@ -446,14 +447,14 @@ static bool bsr_fuse_coupling_plain(Ctx& c, Bsr& B, const Csr& C) {
 }
 
 bool bsr_fuse_coupling(Ctx& c, Bsr& B, const Csr& C) {
+    if (B.fp32) return false;          // the fused kernels read the fp64 values, which fp32 storage released
     return B.t_ok ? bsr_fuse_coupling_tma(c, B, C) : bsr_fuse_coupling_plain(c, B, C);
 }
 
 template <int MODE>
 int bsr_launch(Ctx& c, const Bsr& B, const double* x, double* y, const Epilogue& ep, double* dot_partial, const double* x2) {
     if (B.t_ok) return bsr_tma_launch<MODE>(c, B, x, y, ep, dot_partial, x2);
-    const double a = B.nbrows ? (double)B.nnzb / B.nbrows : 0.0;
-    const int G = a <= 1.5 ? 1 : a <= 4 ? 2 : a <= 12 ? 4 : a <= 48 ? 8 : a <= 160 ? 16 : 32;
+    const int G = row_group_lanes(B.nbrows ? (double)B.nnzb / B.nbrows : 0.0);
     const bool fuse = x2 != nullptr && B.fused;
     const BsrPrefetch pf{B.pf_groups, (int)(B.nnzb >> 5), B.pf_rows, B.nbrows * B.bs};
 #define GO(BSS, DG, PF, FS)                                                                                                     \

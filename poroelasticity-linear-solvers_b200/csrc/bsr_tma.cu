@@ -110,10 +110,13 @@ k_bsr_tma(const int4* __restrict__ desc, int nchunk, const int* __restrict__ crp
         const uint32_t groups = (cnt + 31u) >> 5;
         const uint32_t vb = groups * NE * 256u, cb = groups * 128u, rb = ((nbr + 1u + 3u) >> 2) * 16u, mb = FUSE ? groups * 256u : 0u;
         mbar_expect_tx(&bars[st], vb + cb + rb + mb);
-        bulk_g2s(base, val + (size_t)(d.y >> 5) * NE * 32, vb, &bars[st], policy);
-        bulk_g2s(base + L::VAL_BYTES, col + d.y, cb, &bars[st], policy);
+        // a chunk of >= 64 empty block rows has no blocks: no zero-byte copies (the row pointers, rb >= 16, still arrive)
+        if (cnt) {
+            bulk_g2s(base, val + (size_t)(d.y >> 5) * NE * 32, vb, &bars[st], policy);
+            bulk_g2s(base + L::VAL_BYTES, col + d.y, cb, &bars[st], policy);
+            if (FUSE) bulk_g2s(base + L::VAL_BYTES + L::COL_BYTES + L::RP_BYTES, mval + d.y, mb, &bars[st], policy);
+        }
         bulk_g2s(base + L::VAL_BYTES + L::COL_BYTES, crp + d.z, rb, &bars[st], policy);
-        if (FUSE) bulk_g2s(base + L::VAL_BYTES + L::COL_BYTES + L::RP_BYTES, mval + d.y, mb, &bars[st], policy);
     };
     if (tid == 0)
         for (int k = 0; k < kStages && k < nloc; ++k) issue(k);
@@ -405,8 +408,7 @@ static void launch_one(Ctx& c, const Bsr& B, const double* x, const double* x2, 
 
 template <int MODE>
 int bsr_tma_launch(Ctx& c, const Bsr& B, const double* x, double* y, const Epilogue& ep, double* dot_partial, const double* x2) {
-    const double a = B.nbrows ? (double)B.nnzb / B.nbrows : 0.0;
-    const int G = a <= 1.5 ? 1 : a <= 4 ? 2 : a <= 12 ? 4 : a <= 48 ? 8 : a <= 160 ? 16 : 32;
+    const int G = row_group_lanes(B.nbrows ? (double)B.nnzb / B.nbrows : 0.0);
     const bool fuse = x2 != nullptr && B.t_fused;
     const int min_b = B.t_cfg == 0 ? 2 : (B.t_cfg == 1 ? 4 : 3);
     const int grid = std::min(B.t_nchunk, min_b * c.sm_count);

@@ -33,6 +33,7 @@ struct poro_mat {
     poro_ctx* ctx;
     Csr raw;
     DBuf<double> xext;
+    int fuse_state = -1;         // poro_mat_mult_fused: -1 not tried, 0 refused, 1 the coupling rides along
 };
 struct poro_pc {
     poro_ctx* ctx;
@@ -179,6 +180,7 @@ int poro_mat_create_csr(poro_ctx* h, int64_t nrows, int64_t ncols, const int64_t
         csr_choose_lanes(A);
     }
     m->raw.block_hint = c.opt_i("-poro_mat_block_hint", 0);   // micro-benchmarks: treat the raw matrix as node-blocked
+    m->raw.fp32_hint = c.opt_i("-poro_mat_fp32_values", 0) != 0;
     *out = m.release();
     API_END
 }
@@ -189,6 +191,7 @@ poro_mat* poro_mat_adopt(poro_ctx* h, Csr&& A) {
     m->ctx = h;
     m->raw = std::move(A);
     m->raw.block_hint = h->c.opt_i("-poro_mat_block_hint", 0);
+    m->raw.fp32_hint = h->c.opt_i("-poro_mat_fp32_values", 0) != 0;
     return m.release();
 }
 Ctx& poro_ctx_ref(poro_ctx* h) { return h->c; }
@@ -231,6 +234,52 @@ int poro_mat_mult(poro_mat* m, const double* x, double* y) {
         xin = m->xext.p;
     }
     spmv(c, m->raw, xin, y);
+    API_END
+}
+
+// one product in epilogue mode `mode` (include/poro.h, poro_pc_block_mult); `op` applies modes 0..2 when given, else B does
+static void mult_in_mode(Ctx& c, const Csr& B, MatOp* op, int mode, const double* x, double* y, const double* z, double* r,
+                         double* d_new, double* xv, const double* dinv, double c1, double c2, double* dot) {
+    PORO_REQUIRE(mode >= 0 && mode <= 4, "mode in 0..4");
+    PORO_REQUIRE(mode <= 2 || B.nrows == B.ncols, "Chebyshev / dot modes need a square matrix");
+    if (mode <= 2 && op) op->apply(x, y, (SpmvMode)mode, z);
+    else if (mode <= 2) spmv(c, B, x, y, (SpmvMode)mode, z);
+    else if (mode == 3) spmv_cheb_step(c, B, x, x, d_new, r, xv, dinv, c1, c2);
+    else spmv_dot(c, B, x, y, dot);
+    PORO_CUDA(cudaStreamSynchronize(c.stream));
+}
+
+int poro_mat_mult_mode(poro_mat* m, int mode, const double* x, double* y, const double* z, double* r, double* d_new, double* xv,
+                       const double* dinv, double c1, double c2, double* dot) {
+    API_BEGIN
+    PORO_REQUIRE(m->ctx->c.nranks == 1, "poro_mat_mult_mode: single rank only");
+    mult_in_mode(m->ctx->c, m->raw, nullptr, mode, x, y, z, r, d_new, xv, dinv, c1, c2, dot);
+    API_END
+}
+
+int poro_mat_kernel_info(poro_mat* m, int64_t* out, int n) {
+    API_BEGIN
+    int64_t v[kSpmvInfoFields];
+    spmv_kernel_info(m->ctx->c, m->raw, v);
+    for (int i = 0; i < n; ++i) out[i] = i < kSpmvInfoFields ? v[i] : 0;
+    API_END
+}
+
+int poro_mat_mult_fused(poro_mat* a, poro_mat* cpl, int mode, const double* x, const double* x2, double* y, const double* z, int* fused) {
+    API_BEGIN
+    Ctx& c = a->ctx->c;
+    const Csr& A = a->raw;
+    const Csr& C = cpl->raw;
+    PORO_REQUIRE(mode >= 0 && mode <= 2, "mode in 0..2");
+    PORO_REQUIRE(C.nrows == A.nrows, "the coupling must have the rows of the matrix");
+    if (a->fuse_state < 0) a->fuse_state = csr_fuse_coupling(c, A, C) ? 1 : 0;
+    if (a->fuse_state == 1) spmv_fused(c, A, x, x2, y, (SpmvMode)mode, z);
+    else {
+        spmv(c, A, x, y, (SpmvMode)mode, z);
+        spmv(c, C, x2, y, mode == SPMV_SET ? SPMV_ADD : (SpmvMode)mode, y);
+    }
+    PORO_CUDA(cudaStreamSynchronize(c.stream));
+    if (fused) *fused = a->fuse_state;
     API_END
 }
 
@@ -816,14 +865,7 @@ int poro_pc_block_mult(poro_pc* pc, const char* name, int mode, const double* x,
     API_BEGIN
     MatOp* m = find_block(pc, name);
     if (!m) throw Error(std::string("no such block: ") + name);
-    Ctx& c = pc->ctx->c;
-    const Csr& B = m->mat();
-    PORO_REQUIRE(mode >= 0 && mode <= 4, "mode in 0..4");
-    PORO_REQUIRE(mode <= 2 || B.nrows == B.ncols, "Chebyshev / dot modes need a square block");
-    if (mode <= 2) m->apply(x, y, (SpmvMode)mode, z);
-    else if (mode == 3) spmv_cheb_step(c, B, x, x, d_new, r, xv, dinv, c1, c2);
-    else spmv_dot(c, B, x, y, dot);
-    PORO_CUDA(cudaStreamSynchronize(c.stream));
+    mult_in_mode(pc->ctx->c, m->mat(), m, mode, x, y, z, r, d_new, xv, dinv, c1, c2, dot);
     API_END
 }
 

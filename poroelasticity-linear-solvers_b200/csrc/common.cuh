@@ -296,6 +296,9 @@ bool csr_ensure_bsr(Ctx& c, const Csr& A);
 // spmv_fused(A, x, x2, ...) computes A x + C x2 in one pass over A's blocks
 bool csr_fuse_coupling(Ctx& c, const Csr& A, const Csr& C);
 void spmv_fused(Ctx& c, const Csr& A, const double* x, const double* x2, double* y, SpmvMode mode = SPMV_SET, const double* z = nullptr);
+// what the next product with A launches, after the conversion it would do (fields: include/poro.h, poro_mat_kernel_info)
+constexpr int kSpmvInfoFields = 11;
+void spmv_kernel_info(Ctx& c, const Csr& A, int64_t* v);
 // fused Chebyshev step: t = A d_old; r -= t; d_new = c1 d_old + c2 dinv.*r; x += d_new
 void spmv_cheb_step(Ctx& c, const Csr& A, const double* x_in, const double* d_old, double* d_new, double* r, double* x,
                     const double* dinv, double c1, double c2);

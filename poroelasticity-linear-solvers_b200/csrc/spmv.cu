@@ -208,8 +208,7 @@ static int launch_spmv(Ctx& c, const Csr& A, const double* x, double* y, const E
     int grid;
     if (A.nblk > 0) {
         grid = A.nblk;
-        const double a = A.avg_row();
-        const int G = a <= 1.5 ? 1 : a <= 4 ? 2 : a <= 12 ? 4 : a <= 48 ? 8 : a <= 160 ? 16 : 32;
+        const int G = row_group_lanes(A.avg_row());
 #define GO(GG) k_spmv_stream<GG, MODE><<<grid, kSpmvBlock, 0, c.stream>>>(reinterpret_cast<const int4*>(A.blk_row.p), A.rowptr.p, A.col.p, A.val.p, x, y, ep, dot_partial)
         switch (G) {
             case 1: GO(1); break;
@@ -235,6 +234,36 @@ static int launch_spmv(Ctx& c, const Csr& A, const double* x, double* y, const E
     }
     PORO_LAUNCH_CHECK(c);
     return grid;
+}
+
+void spmv_kernel_info(Ctx& c, const Csr& A, int64_t* v) {
+    std::fill(v, v + kSpmvInfoFields, (int64_t)0);
+    v[7] = -1;
+    if (A.stencil && A.stencil->fr >= 0) { v[0] = 4; return; }
+    if (A.nrows > 0 && csr_ensure_bsr(c, A)) {
+        const Bsr& B = *A.bsr;
+        const bool plain = !B.t_ok;
+        v[0] = B.diag_only ? 2 : 1;
+        v[1] = row_group_lanes(B.nbrows ? (double)B.nnzb / B.nbrows : 0.0);
+        v[2] = B.bs;
+        v[3] = plain && B.pref;
+        v[4] = plain && B.coop && !B.fp32;      // bsr_launch has no cooperative variant for fp32 values
+        v[5] = B.fp32;
+        v[6] = B.t_ok;
+        v[7] = B.t_ok ? B.t_cfg : -1;
+        v[8] = B.t_ok ? B.t_fused : B.fused;
+        v[9] = B.t_ok ? B.t_nchunk : B.nblk;
+        v[10] = plain && B.pf_groups > 0;
+        return;
+    }
+    if (A.nrows > 0 && A.nblk < 0) build_row_blocks(c, A);
+    if (A.nrows == 0 || A.nblk > 0) {
+        v[1] = row_group_lanes(A.avg_row());
+        v[9] = std::max(A.nblk, 0);
+    } else {
+        v[0] = 5;
+        v[1] = A.lanes ? A.lanes : 32;
+    }
 }
 
 void spmv(Ctx& c, const Csr& A, const double* x, double* y, SpmvMode mode, const double* z) {

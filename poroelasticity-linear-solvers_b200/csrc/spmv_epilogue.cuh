@@ -30,6 +30,11 @@ __device__ __forceinline__ double apply_epilogue(const Epilogue& ep, int row, do
     return 0.0;
 }
 
+// lanes that reduce one row (CSR stream) or one block row (BSR), from the average row length in nonzeros or blocks
+inline int row_group_lanes(double avg_row) {
+    return avg_row <= 1.5 ? 1 : avg_row <= 4 ? 2 : avg_row <= 12 ? 4 : avg_row <= 48 ? 8 : avg_row <= 160 ? 16 : 32;
+}
+
 __device__ __forceinline__ double block_sum_256(double v, double* sm) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
