@@ -45,7 +45,13 @@ def build(block: str, N: int, overrides=None, assemble="device", ctx=None, optio
     host = None
     if assemble == "device":
         from poro_b200.generator import generate_swelling3d
-        g = generate_swelling3d(ctx, N, "diagonal", overrides=ov)
+        # `-<prefix>pc_type mg` on the block: attach every coarse level N allows (halving while N stays even)
+        prefixes = ("s_",) if block == "s" else ("fp_fieldsplit_0_",)
+        mg_levels = 1
+        if any(str(ctx.get_option("-" + p + "pc_type", "")) == "mg" for p in prefixes):
+            while N % (1 << mg_levels) == 0:
+                mg_levels += 1
+        g = generate_swelling3d(ctx, N, "diagonal", overrides=ov, mg_levels=mg_levels)
         A, b, imap, par, bcs_p = g.A, g.b, g.index_set(), g.par, g.bcs_sub_pressure
         ns, nf, npp = g.layout.n_field
     else:

@@ -102,6 +102,11 @@ typedef struct poro_gen_table {
 } poro_gen_table;
 int poro_gen_matrix(poro_ctx* ctx, int dim, int N, const poro_gen_table* tables, const int64_t* layout,
                     const uint8_t* bc_flags_host, poro_mat** out);
+/* makes `coarse` the next geometric level of `fine` for `-<prefix>pc_type mg`.  Both come from poro_gen_matrix on one rank
+ * with the same dim, the same present tables, the same lattice kinds and block sizes per field, and N_fine = 2 N_coarse;
+ * anything else fails naming what differs.  `coarse` may have its own coarse level.  `fine` keeps its own reference to the
+ * coarse matrix, so destroying the coarse handle afterwards is safe. */
+int poro_mat_set_coarse(poro_mat* fine, poro_mat* coarse);
 
 /* ---- halo plan for row-partitioned runs (MatMult_MPIAIJ's VecScatter in the reference) ---
  * neighbours k = 0..nneigh-1: this rank sends x[send_idx[send_ptr[k]..send_ptr[k+1])] (owned,
@@ -195,6 +200,15 @@ int poro_pc_amg_info(poro_pc* pc, const char* name, int64_t* rows, int64_t* nnz,
  * largest front, perturbed pivots, device bytes held after set-up, flops of the numeric factorisation, its device time
  * in microseconds, algorithmic bytes of one application without refinement.  Fails for a block that is not a sparse LU. */
 int poro_pc_factor_info(poro_pc* pc, const char* name, int64_t* out, int n);
+/* geometric multigrid of a block's inner PC (`-<prefix>pc_type mg`).  out[0..n) receives the number G of geometric levels
+ * (the finest included), then per geometric level N, rows and the launch format of its operator (4 = stencil), then the
+ * number of algebraic levels below.  Fails for an inner PC that is not `mg`. */
+int poro_pc_mg_info(poro_pc* pc, const char* name, int64_t* out, int n);
+/* one geometric transfer between level `level` and `level + 1` on device vectors: dir 0 prolongation (x coarse, y fine;
+ * mode 0 y = P~ x, mode 1 y += P~ x), dir 1 restriction (x fine, y coarse, y = P~^T x, mode 0) */
+int poro_pc_mg_transfer(poro_pc* pc, const char* name, int level, int dir, int mode, const double* x_dev, double* y_dev);
+/* algorithmic bytes of the transfers of `level`: out[0] prolongation (set), out[1] prolongation (add), out[2] restriction */
+int poro_pc_mg_bytes(poro_pc* pc, const char* name, int level, int64_t* out);
 /* live profile of the outer operator product (the dominant SpMV): CUDA events recorded on the
  * launching stream around every y = A x inside poro_ksp_solve.  enable = 1 resets and starts,
  * 0 stops, -1 only reads.  op_bytes = algorithmic bytes of one product

@@ -41,6 +41,7 @@ SIGNATURES = {
     "poro_mat_kernel_info": [vp, c_i64p, C.c_int],
     "poro_mat_mult_fused": [vp, vp, C.c_int, vp, vp, vp, vp, C.POINTER(C.c_int)],
     "poro_gen_matrix": [vp, C.c_int, C.c_int, vp, vp, vp, C.POINTER(vp)],
+    "poro_mat_set_coarse": [vp, vp],
     "poro_halo_set": [vp, C.c_int64, C.c_int, vp, vp, vp, vp],
     "poro_fields_set": [vp, vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int, C.c_int],
     "poro_fields_set_coords": [vp, C.c_int, vp, vp],
@@ -70,6 +71,9 @@ SIGNATURES = {
     "poro_pc_inner_solve": [vp, C.c_char_p, vp, vp],
     "poro_pc_amg_info": [vp, C.c_char_p, c_i64p, c_i64p, C.c_int, C.POINTER(C.c_int)],
     "poro_pc_factor_info": [vp, C.c_char_p, c_i64p, C.c_int],
+    "poro_pc_mg_info": [vp, C.c_char_p, c_i64p, C.c_int],
+    "poro_pc_mg_transfer": [vp, C.c_char_p, C.c_int, C.c_int, C.c_int, vp, vp],
+    "poro_pc_mg_bytes": [vp, C.c_char_p, C.c_int, c_i64p],
     "poro_ksp_mult": [vp, vp, vp],
     "poro_ksp_profile": [vp, C.c_int, c_f64p, c_i64p, c_i64p],
     "poro_profile": [vp, C.c_int, c_f64p, c_i64p, C.c_int],

@@ -9,7 +9,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libporo.so")
-SOURCES = ["vec.cu", "spmv.cu", "stencil.cu", "bsr.cu", "bsr_tma.cu", "setup.cu", "amg.cu", "distamg.cu", "solver.cu", "sparse_lu.cu", "dist.cu", "gen.cu", "capi.cu"]
+SOURCES = ["vec.cu", "spmv.cu", "stencil.cu", "mg.cu", "bsr.cu", "bsr_tma.cu", "setup.cu", "amg.cu", "distamg.cu", "solver.cu", "sparse_lu.cu", "dist.cu", "gen.cu", "capi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "--extended-lambda",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default", "-Xptxas", "-v" if os.environ.get("PORO_PTXAS_V") else "-O3"]

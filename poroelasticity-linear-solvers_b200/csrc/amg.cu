@@ -492,7 +492,9 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
                     (long long)Acur->nnz, bs, Lp->lmax, dist ? " distributed" : "");
         Lp->x.alloc((size_t)n + n_gh); Lp->b.alloc(n); Lp->r.alloc((size_t)n + n_gh); Lp->d0.alloc((size_t)n + n_gh); Lp->d1.alloc((size_t)n + n_gh);
         if (dist) Lp->ext.alloc((size_t)n + n_gh);
-        if (n_glob <= par.coarse_size || (int)levels.size() >= par.max_levels) break;
+        // geometric levels are taken whatever their size; the algebraic ones count from the coarsest geometric level
+        const bool geo_next = (int)levels.size() < par.mg_levels;
+        if (!geo_next && (n_glob <= par.coarse_size || (int)levels.size() - std::max(par.mg_levels - 1, 0) >= par.max_levels)) break;
         // Dirichlet rows (diagonal only) carry no near-nullspace
         {
             const int* rp = Acur->rowptr.p; const int* cc = Acur->col.p; const double* v = Acur->val.p;
@@ -502,6 +504,22 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
                 for (int q = rp[i]; q < rp[i + 1]; ++q) { if (cc[q] == (int)i) d += v[q]; else off += fabs(v[q]); }
                 if (off <= 1e-14 * fabs(d)) for (int j = 0; j < kk; ++j) b[(size_t)i * kk + j] = 0.0;
             });
+        }
+        if (geo_next) {
+            // the same block generated at N/2 (rediscretisation = Galerkin product with the geometric transfer), the
+            // near-nullspace injected at the coinciding nodes (exact for the rigid-body modes: the coarse space holds them)
+            Tick t(c, "geometric level");
+            Csr Ac;
+            mg_coarse_block(c, *Acur->stencil, Ac);
+            Ac.block_hint = bs;
+            Lp->mg = std::make_unique<MgTransfer>();
+            mg_transfer_init(c, *Lp->mg, *Acur->stencil, *Ac.stencil);
+            DBuf<double> Bc;
+            mg_inject(c, *Lp->mg, B.p, k, Bc);
+            Anext = std::move(Ac);
+            have_next = true;
+            B = std::move(Bc);
+            continue;
         }
         // aggregation sees the owned diagonal block only: aggregates never cross a rank boundary
         Csr sq;
@@ -712,9 +730,11 @@ void Amg::cycle(int l, const double* b, double* x) {
     AmgLevel& Ln = *levels[l + 1];
     cheby(l, b, x, true);
     spmv(c, A, ext(l, x), L.r.p, SPMV_SUB, b);
-    spmv(c, L.R, ext(l, L.r.p), Ln.b.p);                               // restriction reads the ghost residuals
+    if (L.mg) mg_restrict(c, *L.mg, L.r.p, Ln.b.p);
+    else spmv(c, L.R, ext(l, L.r.p), Ln.b.p);                          // restriction reads the ghost residuals
     cycle(l + 1, Ln.b.p, Ln.x.p);
-    spmv(c, L.P, ext(l + 1, Ln.x.p), x, SPMV_ADD, x);                  // prolongation reads the ghost coarse values
+    if (L.mg) mg_prolong(c, *L.mg, Ln.x.p, x, true);
+    else spmv(c, L.P, ext(l + 1, Ln.x.p), x, SPMV_ADD, x);             // prolongation reads the ghost coarse values
     if (par.post_smooth) cheby(l, b, x, false);
 }
 

@@ -1,6 +1,7 @@
 // amg.cuh -- smoothed-aggregation AMG hierarchy (device set-up + V-cycle).
 #pragma once
 #include "common.cuh"
+#include "mg.cuh"
 #include <functional>
 
 namespace poro {
@@ -14,6 +15,9 @@ struct AmgParams {
     int power_its = 15;
     int post_smooth = 1;        // 0: V(nu,0) cycle (non-symmetric: only under GMRES/FGMRES)
     bool smoother_only = false; // `-*_pc_type chebyshev`: one level, no coarse solve of any kind
+    // `-*_pc_type mg`: levels 0 .. mg_levels - 1 are the generated block and its attached coarse levels (geometric transfer,
+    // mg.cuh); the last of them is level 0 of the SA-AMG below, and max_levels counts from there
+    int mg_levels = 0;
 };
 
 struct AmgLevel {
@@ -29,6 +33,7 @@ struct AmgLevel {
     std::unique_ptr<DistPlan> owned_plan;
     bool replicated = false;        // this level and everything below is gathered on every rank and cycled redundantly (Amg::tail)
     DBuf<double> ext;               // staging for vectors that are not stored extended (the caller's x on level 0)
+    std::unique_ptr<MgTransfer> mg; // geometric level: the transfer to the next level replaces P and R
 };
 
 struct Amg {

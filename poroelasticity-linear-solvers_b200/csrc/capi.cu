@@ -237,6 +237,37 @@ int poro_mat_mult(poro_mat* m, const double* x, double* y) {
     API_END
 }
 
+int poro_mat_set_coarse(poro_mat* fine, poro_mat* coarse) {
+    API_BEGIN
+    PORO_REQUIRE(fine && coarse && fine != coarse, "poro_mat_set_coarse: two distinct matrices are needed");
+    PORO_REQUIRE(fine->ctx == coarse->ctx, "poro_mat_set_coarse: the matrices belong to different contexts");
+    const Csr& F = fine->raw;
+    const Csr& G = coarse->raw;
+    auto generated = [](const Csr& M) { return M.stencil && M.stencil->fr < 0; };
+    PORO_REQUIRE(generated(F), "poro_mat_set_coarse: the fine matrix was not generated by poro_gen_matrix on one rank");
+    PORO_REQUIRE(generated(G), "poro_mat_set_coarse: the coarse matrix was not generated by poro_gen_matrix on one rank");
+    const StencilData& f = *F.stencil->d;
+    const StencilData& g = *G.stencil->d;
+    PORO_REQUIRE(f.dim == g.dim, "poro_mat_set_coarse: dim differs (fine " + std::to_string(f.dim) + ", coarse " + std::to_string(g.dim) + ")");
+    PORO_REQUIRE(f.N == 2 * g.N, "poro_mat_set_coarse: N_fine must be 2 N_coarse (fine N = " + std::to_string(f.N) + ", coarse N = " +
+                                     std::to_string(g.N) + ")");
+    for (int b = 0; b < 9; ++b)
+        PORO_REQUIRE(f.present[b] == g.present[b], "poro_mat_set_coarse: the present tables differ (field block " + std::to_string(b / 3) +
+                                                       "," + std::to_string(b % 3) + ")");
+    for (int fld = 0; fld < 3; ++fld)
+        PORO_REQUIRE(f.kind[fld] == g.kind[fld] && f.bdim[fld] == g.bdim[fld],
+                     "poro_mat_set_coarse: lattice kind or block size of field " + std::to_string(fld) + " differs");
+    PORO_REQUIRE((f.bc.p != nullptr) == (g.bc.p != nullptr), "poro_mat_set_coarse: one matrix has Dirichlet flags, the other none");
+    // the fine descriptor keeps its own reference to the coarse matrix: destroying the coarse handle afterwards is safe
+    auto keep = std::make_shared<Csr>();
+    csr_copy(coarse->ctx->c, G, *keep);
+    PORO_CUDA(cudaStreamSynchronize(coarse->ctx->c.stream));
+    csr_choose_lanes(*keep);
+    keep->stencil = G.stencil;
+    F.stencil->d->coarse = std::move(keep);
+    API_END
+}
+
 // one product in epilogue mode `mode` (include/poro.h, poro_pc_block_mult); `op` applies modes 0..2 when given, else B does
 static void mult_in_mode(Ctx& c, const Csr& B, MatOp* op, int mode, const double* x, double* y, const double* z, double* r,
                          double* d_new, double* xv, const double* dinv, double c1, double c2, double* dot) {
@@ -527,7 +558,10 @@ static std::unique_ptr<KSP> make_inner(poro_ctx* h, MatOp* op, const std::string
     std::string pt = c.opt("-" + prefix + "pc_type", pc_type);
     if (pt == "fieldsplit") pt = "amg";
     const Csr* src = &op->mat();
-    const bool amg_type = pt == "hypre" || pt == "amg" || pt == "gamg" || pt == "ml" || pt == "chebyshev";
+    if (pt == "mg" && c.nranks > 1)
+        throw Error("-" + prefix + "pc_type mg: geometric multigrid runs on one rank, this block is row-partitioned over " +
+                    std::to_string(c.nranks) + " ranks");
+    const bool amg_type = pt == "hypre" || pt == "amg" || pt == "gamg" || pt == "ml" || pt == "chebyshev" || pt == "mg";
     // row-partitioned runs: hierarchies are distributed (global Galerkin coarse levels, distamg.cu) whenever the block has
     // ONE halo plan; the decision uses global sizes so that every rank takes the same (collective) path
     DistPlan* plan = nullptr;
@@ -920,6 +954,58 @@ int poro_pc_amg_info(poro_pc* pc, const char* name, int64_t* rows, int64_t* nnz,
     if (!a) { *nlevels = 0; return 0; }
     *nlevels = (int)a->amg.levels.size();
     for (int l = 0; l < *nlevels && l < cap; ++l) { rows[l] = a->amg.op(l).nrows; nnz[l] = a->amg.op(l).nnz; }
+    API_END
+}
+
+static Amg& mg_amg(poro_pc* pc, const char* name) {
+    KSP* k = find_ksp(pc, name ? name : "");
+    if (!k) throw Error(std::string("no such inner solver: ") + (name ? name : ""));
+    PCAmg* a = dynamic_cast<PCAmg*>(k->pc);
+    if (!a || a->amg.par.mg_levels < 1) throw Error(std::string("inner solver '") + name + "' is not a geometric multigrid (pc_type mg)");
+    return a->amg;
+}
+
+int poro_pc_mg_info(poro_pc* pc, const char* name, int64_t* out, int n) {
+    API_BEGIN
+    Amg& a = mg_amg(pc, name);
+    int geo = 1;
+    while (geo < (int)a.levels.size() && a.levels[geo - 1]->mg) ++geo;
+    std::vector<int64_t> v = {geo};
+    for (int l = 0; l < geo; ++l) {
+        const Csr& A = a.op(l);
+        const bool st = A.stencil && A.stencil->fr >= 0;
+        v.push_back(st ? A.stencil->d->N : -1);
+        v.push_back(A.nrows);
+        v.push_back(st ? 4 : 0);
+    }
+    v.push_back((int64_t)a.levels.size() - geo);
+    for (int i = 0; i < n; ++i) out[i] = i < (int)v.size() ? v[i] : 0;
+    API_END
+}
+
+int poro_pc_mg_transfer(poro_pc* pc, const char* name, int level, int dir, int mode, const double* x, double* y) {
+    API_BEGIN
+    Amg& a = mg_amg(pc, name);
+    PORO_REQUIRE(level >= 0 && level < (int)a.levels.size() && a.levels[level]->mg, "poro_pc_mg_transfer: level " + std::to_string(level) +
+                                                                                        " has no geometric transfer");
+    PORO_REQUIRE(dir == 0 || dir == 1, "poro_pc_mg_transfer: dir is 0 (prolongation) or 1 (restriction)");
+    PORO_REQUIRE(mode == 0 || mode == 1, "poro_pc_mg_transfer: mode is 0 (set) or 1 (add)");
+    PORO_REQUIRE(dir == 0 || mode == 0, "poro_pc_mg_transfer: restriction has mode 0 only");
+    Ctx& c = pc->ctx->c;
+    if (dir == 0) mg_prolong(c, *a.levels[level]->mg, x, y, mode == 1);
+    else mg_restrict(c, *a.levels[level]->mg, x, y);
+    API_END
+}
+
+int poro_pc_mg_bytes(poro_pc* pc, const char* name, int level, int64_t* out) {
+    API_BEGIN
+    Amg& a = mg_amg(pc, name);
+    PORO_REQUIRE(level >= 0 && level < (int)a.levels.size() && a.levels[level]->mg, "poro_pc_mg_bytes: level " + std::to_string(level) +
+                                                                                     " has no geometric transfer");
+    const MgTransfer& t = *a.levels[level]->mg;
+    out[0] = mg_prolong_bytes(t, false);
+    out[1] = mg_prolong_bytes(t, true);
+    out[2] = mg_restrict_bytes(t);
     API_END
 }
 

@@ -144,7 +144,23 @@ std::unique_ptr<PC> make_pc(Ctx& c, const std::string& pc_type, const Csr& A, in
     if (!plan && use_sparse_lu(c, pc_type, prefix, A.nrows)) return std::make_unique<PCSparseLU>(&c, A, prefix);
     if (want_lu && !plan && A.nrows <=c.opt_i("-poro_dense_lu_limit", 8192)) return std::make_unique<PCDense>(&c, A);
     const bool cheb_only = pc_type == "chebyshev";      // Chebyshev(degree) on D^-1 A = a one-level hierarchy
-    if (want_lu || cheb_only || pc_type == "hypre" || pc_type == "amg" || pc_type == "gamg" || pc_type == "ml") {
+    const bool mg = pc_type == "mg";                    // geometric levels on top of the SA-AMG (mg.cuh)
+    int mg_levels = 0;
+    if (mg) {
+        const std::string key = "-" + prefix + "pc_type mg";
+        if (plan || c.nranks > 1) throw Error(key + ": geometric multigrid runs on one rank only");
+        if (!A.stencil || A.stencil->fr < 0 || A.stencil->fc != A.stencil->fr)
+            throw Error(key + " needs a single generated field block; this block has no class-stencil descriptor (uploaded "
+                        "through poro_mat_create_csr, permuted, cut across several fields, or a Schur complement)");
+        const int attached = mg_attached_levels(*A.stencil);
+        if (attached == 0)
+            throw Error(key + ": the generated matrix has no coarse levels attached (poro_mat_set_coarse, or mg_levels > 1 in "
+                        "the generator)");
+        mg_levels = c.opt_i("-" + prefix + "pc_mg_levels", attached + 1);
+        if (mg_levels < 1) throw Error("-" + prefix + "pc_mg_levels must be at least 1");
+        mg_levels = std::min(mg_levels, attached + 1);
+    }
+    if (want_lu || cheb_only || mg || pc_type == "hypre" || pc_type == "amg" || pc_type == "gamg" || pc_type == "ml") {
         auto pc = std::make_unique<PCAmg>();
         AmgParams p;
         p.theta = c.opt_d("-" + prefix + "pc_amg_theta", c.opt_d("-pc_amg_theta", p.theta));
@@ -159,6 +175,7 @@ std::unique_ptr<PC> make_pc(Ctx& c, const std::string& pc_type, const Csr& A, in
             p.max_levels = 1;
             p.cheby_degree = c.opt_i("-" + prefix + "pc_amg_cheby_degree", 4);
         }
+        p.mg_levels = mg_levels;
         bool use_rbm = c.opt_i("-" + prefix + "pc_amg_rigid_body_modes", c.opt_i("-pc_amg_rigid_body_modes", 1)) != 0;
         if (bs > 1 && coords_host && coord_dim == bs && use_rbm) {
             std::vector<double> B;

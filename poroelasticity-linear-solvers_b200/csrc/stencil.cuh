@@ -30,6 +30,9 @@ struct StencilData {
     // warp has the same class, so table reads are broadcasts and no warp diverges on the entry count
     DBuf<int2> wdesc[2];
     int nwarps[2] = {0};
+    // next geometric level (poro_mat_set_coarse): the same matrix generated at N / 2, shared with its handle; its own
+    // descriptor may link further down (mg.cuh)
+    std::shared_ptr<const Csr> coarse;
 };
 
 // the operator of a Csr: row field `fr` against column field `fc` (a block extracted along whole fields), or against all

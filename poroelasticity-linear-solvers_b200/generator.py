@@ -234,10 +234,91 @@ class GeneratedSystem:
                         coords_p=self.coords_p)
 
 
+class WholeLayout:
+    """Single-rank layout of the whole unit square or cube: every node owned, no ghosts, fields [s | f | p]."""
+
+    def __init__(self, dim: int, N: int):
+        L2, L1 = 2 * N + 1, N + 1
+        self.dim, self.N = dim, N
+        self.n2, self.n1 = L2 ** dim, L1 ** dim
+        self.n_field = [dim * self.n2, dim * self.n2, self.n1]
+        self.off_owned = [0, self.n_field[0], self.n_field[0] + self.n_field[1]]
+        self.n_owned = self.n_ext = sum(self.n_field)
+
+    def layout_array(self) -> np.ndarray:
+        o = self.n_owned
+        return np.asarray([0, self.n1, 0, 0, 0, 0, 0, self.n2, 0, 0, 0, 0, *self.off_owned, o, o, o, o, o, o, o], np.int64)
+
+
+def _check_mg_levels(N: int, mg_levels: int, world: int = 1):
+    if mg_levels < 1:
+        raise ValueError("mg_levels must be at least 1, got %d" % mg_levels)
+    if mg_levels > 1 and world != 1:
+        raise ValueError("geometric coarse levels (mg_levels > 1) are generated on one rank only, not on %d" % world)
+    if N % (1 << (mg_levels - 1)):
+        raise ValueError("N = %d is not divisible by 2^(mg_levels - 1) = %d" % (N, 1 << (mg_levels - 1)))
+
+
+def _swelling_operators(ctx, dim: int, N: int, pc_type: str, overrides, layout, p2_range=None, p1_range=None):
+    """A, P, P_diff of the swelling problem on `layout` (the node ranges select the owned flags; default: all nodes)."""
+    from hostfem.stencil import swelling_generator
+    gen, par, loads = swelling_generator(dim, N, overrides)
+    bc_s = gen.bc_s[slice(*p2_range) if p2_range else slice(None)].ravel()
+    bc_f = gen.bc_f[slice(*p2_range) if p2_range else slice(None)].ravel()
+    bc_p = gen.bc_p[slice(*p1_range) if p1_range else slice(None)]
+    flags = np.concatenate([bc_s, bc_f, np.zeros(len(bc_p), bool)])   # pressure BCs only go to P_diff (lib/Poromechanics.py:76-83)
+    A = generate_matrix(ctx, gen, layout, "A", pc_type, flags)
+    P = generate_matrix(ctx, gen, layout, "P", pc_type, flags)
+    Pd = None
+    if "3-way" in pc_type:
+        Pd = generate_matrix(ctx, gen, layout, "P_diff", pc_type, np.concatenate([bc_s, bc_f, bc_p]))
+    return A, P, Pd, gen, par, loads
+
+
+def _attach_coarse_levels(ctx, dim: int, N: int, pc_type: str, overrides, mg_levels: int, ops):
+    """Generates A, P, P_diff at N/2, N/4, ... (mg_levels - 1 levels) and links each fine matrix of `ops` to its coarse
+    chain (poro_mat_set_coarse).  The fine matrices keep the coarse ones alive; the coarse handles are released."""
+    chains = [[m] for m in ops]
+    for lev in range(1, mg_levels):
+        Nc = N >> lev
+        A, P, Pd, _, _, _ = _swelling_operators(ctx, dim, Nc, pc_type, overrides, WholeLayout(dim, Nc))
+        for ch, m in zip(chains, (A, P, Pd)):
+            ch.append(m)
+    for ch in chains:
+        if ch[0] is None:
+            continue
+        for i in range(len(ch) - 2, -1, -1):                       # bottom up: every coarse level already has its chain
+            _capi.check(ctx.lib.poro_mat_set_coarse(ch[i].handle, ch[i + 1].handle))
+        for m in ch[1:]:
+            m.destroy()
+
+
+def generate_swelling2d(ctx, N: int, pc_type: str = "diagonal", overrides: dict | None = None, mg_levels: int = 1) -> GeneratedSystem:
+    """swelling.py on the unit square (x 1e-2) with N cells per side, generated on the device on one rank.  mg_levels > 1
+    also generates the operators at N/2, N/4, ... and links them as geometric levels (`-<prefix>pc_type mg`)."""
+    _check_mg_levels(N, mg_levels)
+    lay = WholeLayout(2, N)
+    ctx.set_halo(0, [], [0], [], [])
+    A, P, Pd, gen, par, loads = _swelling_operators(ctx, 2, N, pc_type, overrides, lay)
+    _attach_coarse_levels(ctx, 2, N, pc_type, overrides, mg_levels, (A, P, Pd))
+    par = dict(par)
+    par["pc type"] = pc_type
+    b = gen.rhs(par["t0"] + par["dt"], **loads)
+    o = lay.off_owned
+    is_s, is_f, is_p = (o[f] + np.arange(lay.n_field[f], dtype=np.int64) for f in range(3))
+    c2, c1 = gen.coords(2), gen.coords(1)
+    plan = HaloPlan(lay.n_owned, np.zeros(0, np.int32), np.zeros(1, np.int64), np.zeros(0, np.int32), np.zeros(0, np.int64),
+                    np.zeros(0, np.int64))
+    return GeneratedSystem(2, A, P, Pd, b, is_s, is_f, is_p, np.flatnonzero(gen.bc_p).astype(np.int64), np.repeat(c2, 2, axis=0), c1,
+                           np.arange(lay.n_owned, dtype=np.int64), plan, lay, lay.n_owned, par)
+
+
 def generate_swelling3d(ctx, N: int, pc_type: str = "diagonal", rank: int = 0, world: int = 1, overrides: dict | None = None,
-                        init_dist: bool = True) -> GeneratedSystem:
-    """swelling-3d.py on the unit cube (x 1e-2) with N cells per side: this rank's slab, generated on the device."""
+                        init_dist: bool = True, mg_levels: int = 1) -> GeneratedSystem:
+    """swelling-3d.py on the unit cube (x 1e-2) with N cells per side: this rank's slab, generated on the device.
+    mg_levels > 1 (one rank) also generates the operators at N/2, N/4, ... and links them as geometric levels."""
     from hostfem.stencil import swelling_generator      # element matrices of ONE macro cell + loads (FEniCS stand-in)
+    _check_mg_levels(N, mg_levels, world)
     gen, par, loads = swelling_generator(3, N, overrides)
     par = dict(par)
     par["pc type"] = pc_type
@@ -259,6 +340,7 @@ def generate_swelling3d(ctx, N: int, pc_type: str = "diagonal", rank: int = 0, w
     Pd = None
     if "3-way" in pc_type:
         Pd = generate_matrix(ctx, gen, lay, "P_diff", pc_type, np.concatenate([bc_s, bc_f, bc_p]))
+    _attach_coarse_levels(ctx, 3, N, pc_type, overrides, mg_levels, (A, P, Pd))
     t = par["t0"] + par["dt"]
     b = gen.rhs(t, **loads)[lay.owned_global()]
     is_s, is_f, is_p = lay.index_sets()

@@ -102,6 +102,25 @@ class PreconditionerCC(object):
         _capi.check(self.ctx.lib.poro_pc_factor_info(self.h, name.encode(), out, len(out)))
         return dict(zip(self.FACTOR_INFO_KEYS, (int(v) for v in out)))
 
+    def mg_info(self, name):
+        """Geometric multigrid of an inner PC (`-<prefix>pc_type mg`): ([(N, rows, format) per geometric level, finest
+        first], number of algebraic levels below); raises for an inner PC that is not `mg`."""
+        out = (C.c_int64 * 64)()
+        _capi.check(self.ctx.lib.poro_pc_mg_info(self.h, name.encode(), out, len(out)))
+        g = int(out[0])
+        return [tuple(int(v) for v in out[1 + 3 * l: 4 + 3 * l]) for l in range(g)], int(out[1 + 3 * g])
+
+    def mg_transfer(self, name, level, direction, mode, x, y):
+        """One geometric transfer between `level` and `level + 1` (direction 0: y = / += P~ x, 1: y = P~^T x)."""
+        _capi.check(self.ctx.lib.poro_pc_mg_transfer(self.h, name.encode(), level, direction, mode, _capi._ptr(_tensor(x)),
+                                                     _capi._ptr(_tensor(y))))
+
+    def mg_bytes(self, name, level):
+        """Algorithmic bytes of the transfers of `level`: (prolongation set, prolongation add, restriction)."""
+        out = (C.c_int64 * 3)()
+        _capi.check(self.ctx.lib.poro_pc_mg_bytes(self.h, name.encode(), level, out))
+        return tuple(int(v) for v in out)
+
     def inner_solve(self, name, r, z):
         _capi.check(self.ctx.lib.poro_pc_inner_solve(self.h, name.encode(), _capi._ptr(_tensor(r)), _capi._ptr(_tensor(z))))
 
