@@ -83,6 +83,12 @@ int poro_mat_mult_fused(poro_mat* a, poro_mat* c, int mode, const double* x, con
                         int* fused);
 
 int poro_mat_copy(poro_mat* m, int64_t* rowptr, int32_t* col, double* val);
+/* the set-up primitives on raw matrices (tests): op "spgemm" (a b), "transpose" (a^T) or "add_scaled"
+ * (a + alpha diag(s) b, s a device vector or NULL for ones); *out is a new matrix, *chunks the SpGEMM's row chunks under
+ * -poro_spgemm_chunk (0 for the other ops).  poro_dense_inverse: the Gauss-Jordan inverse of the coarsest AMG level of a
+ * row-major n x n host matrix. */
+int poro_mat_setup_op(poro_mat* a, poro_mat* b, const char* op, double alpha, const double* s_dev, poro_mat** out, int* chunks);
+int poro_dense_inverse(poro_ctx* ctx, int n, const double* a_host, double* inv_host);
 
 /* ---- device-side generator of the assembled system (SURVEY 8 f1) ------------------------------------
  * Replaces the host assembly + DirichletBC.apply of lib/Assembler.py:66-221, lib/Poromechanics.py:76-83 on dolfin's
@@ -194,6 +200,18 @@ int poro_pc_inner_solve(poro_pc* pc, const char* name, const double* r_dev, doub
 int poro_pc_inner_result(poro_pc* pc, const char* name, int* its, int* reason, double* rnorm);
 /* AMG hierarchy of a block's inner PC: per level rows and nnz; returns number of levels */
 int poro_pc_amg_info(poro_pc* pc, const char* name, int64_t* rows, int64_t* nnz, int cap, int* nlevels);
+/* one level of a block's single-rank AMG hierarchy (tests of the set-up).  out[0..n) receives: rows, columns and nnz of
+ * A_l, P_l, R_l and T_l (the tentative prolongator; zeros unless kept), block size, near-nullspace modes k, aggregates,
+ * geometric level, coarsest level, coarsest level solved directly, set-up data kept, and the row chunks of the SpGEMMs
+ * A T, A P and R (A P); *lmax receives the Chebyshev bound 1.1 lambda_max(D^-1 A_l).  `-poro_amg_keep_setup 1` before the
+ * set-up keeps per level the aggregates, the near-nullspace as the level used it (after the Dirichlet zeroing; the
+ * coarsest level's as received) and T_l.  Row-partitioned hierarchies and levels out of range are refused. */
+int poro_pc_amg_level_info(poro_pc* pc, const char* name, int level, int64_t* out, int n, double* lmax);
+/* copy of one item of that level to host arrays sized from poro_pc_amg_level_info: "A" "P" "R" "T" as CSR; "agg" (int32,
+ * in col); "B" (n x k row-major), "dinv" (n) and "inv" (the coarsest dense inverse, n x n row-major) in val.  Refused
+ * with the reason: set-up data not kept (agg B T), a geometric level (P R T agg), the coarsest level (P R T agg), no
+ * direct coarsest solve (inv), a row-partitioned hierarchy, a level out of range. */
+int poro_pc_amg_level_copy(poro_pc* pc, const char* name, int level, const char* what, int64_t* rowptr, int32_t* col, double* val);
 /* sparse LU of a block's inner PC ("s","f","p","fp","diff"; -<prefix>pc_factor_mat_solver_type poro above
  * -poro_dense_lu_limit rows).  out[0..n) receives, in this order: rows, nnz(L) (strictly lower), nnz(U) (with the
  * diagonal), explicit zeros stored by supernode amalgamation, supernodes, levels of the supernodal tree, rows of the

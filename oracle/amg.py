@@ -57,9 +57,22 @@ def rigid_body_modes(coords: np.ndarray, dim: int) -> np.ndarray:
 def strength_graph(A: sp.csr_matrix, bs: int, theta: float):
     """Symmetrised nodal strength graph (CSR pattern + weights = block Frobenius norms^2)."""
     nn = A.shape[0] // bs
-    C = A.tocoo()
-    N2 = sp.coo_matrix((C.data ** 2, (C.row // bs, C.col // bs)), shape=(nn, nn)).tocsr()
-    N2.sum_duplicates()
+    C = sp.csr_matrix(A).tocoo()
+    # each block's squares summed one after the other in stored order, as amg.cu's segmented combine does: the weights are
+    # then bit-equal to the device's, so a tie between neighbours is broken the same way on both sides
+    key = (C.row // bs).astype(np.int64) * nn + C.col // bs
+    order = np.argsort(key, kind="stable")
+    key, sq = key[order], C.data[order] ** 2
+    head = np.ones(len(key), bool)
+    head[1:] = key[1:] != key[:-1]
+    seg = np.cumsum(head) - 1
+    start = np.flatnonzero(head)
+    w = np.zeros(len(start))
+    pos = np.arange(len(key)) - start[seg]
+    for t in range(int(pos.max()) + 1 if len(pos) else 0):
+        sel = pos == t
+        w[seg[sel]] += sq[sel]
+    N2 = sp.csr_matrix((w, (key[head] // nn, key[head] % nn)), shape=(nn, nn))
     d = N2.diagonal()
     G = N2.tocoo()
     strong = (G.row != G.col) & (G.data >= theta * theta * np.sqrt(d[G.row] * d[G.col])) & (G.data > 0)
@@ -169,10 +182,12 @@ class Level:
 
 
 class SAAMG:
+    post_smooth = True              # False: V(nu, 0) cycle (amg.cu: -*_pc_amg_post_smooth 0)
+
     def __init__(self, A: sp.csr_matrix, bs: int = 1, B: np.ndarray | None = None, theta: float = 0.08,
                  max_levels: int = 10, coarse_size: int = 400, cheby_degree: int = 2, cheby_ratio: float = 10.0,
                  power_its: int = 15, dense_limit: int = 4096, node_labels: np.ndarray | None = None,
-                 local_smoothing: bool = False):
+                 local_smoothing: bool = False, post_smooth: bool = True):
         """node_labels (one int per node): aggregates never cross a label boundary ("uncoupled" aggregation
         of a row-partitioned matrix: each rank aggregates its own nodes) while smoothing of P and the Galerkin
         product stay global.  The coarse nodes inherit the label of their aggregate."""
@@ -186,7 +201,7 @@ class SAAMG:
                 B[c::bs, c] = 1.0
         B = B.copy()
         self.levels = []
-        self.deg, self.ratio = cheby_degree, cheby_ratio
+        self.deg, self.ratio, self.post_smooth = cheby_degree, cheby_ratio, post_smooth
         while True:
             L = Level()
             L.A = A
@@ -280,7 +295,7 @@ class SAAMG:
         r = b - L.A @ x
         xc = self._cycle(l + 1, L.R @ r)
         x = x + L.P @ xc
-        return self._cheby(L, b, x, False)
+        return self._cheby(L, b, x, False) if self.post_smooth else x
 
     def __call__(self, b):
         return self._cycle(0, b)

@@ -37,6 +37,8 @@ SIGNATURES = {
     "poro_mat_mult": [vp, vp, vp],
     "poro_mat_bench": [vp, C.c_int, C.c_int, c_f64p],
     "poro_mat_copy": [vp, vp, vp, vp],
+    "poro_mat_setup_op": [vp, vp, C.c_char_p, C.c_double, vp, C.POINTER(vp), C.POINTER(C.c_int)],
+    "poro_dense_inverse": [vp, C.c_int, vp, vp],
     "poro_mat_mult_mode": [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_double, C.c_double, vp],
     "poro_mat_kernel_info": [vp, c_i64p, C.c_int],
     "poro_mat_mult_fused": [vp, vp, C.c_int, vp, vp, vp, vp, C.POINTER(C.c_int)],
@@ -70,6 +72,8 @@ SIGNATURES = {
     "poro_pc_block_mult": [vp, C.c_char_p, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_double, C.c_double, vp],
     "poro_pc_inner_solve": [vp, C.c_char_p, vp, vp],
     "poro_pc_amg_info": [vp, C.c_char_p, c_i64p, c_i64p, C.c_int, C.POINTER(C.c_int)],
+    "poro_pc_amg_level_info": [vp, C.c_char_p, C.c_int, c_i64p, C.c_int, c_f64p],
+    "poro_pc_amg_level_copy": [vp, C.c_char_p, C.c_int, C.c_char_p, vp, vp, vp],
     "poro_pc_factor_info": [vp, C.c_char_p, c_i64p, C.c_int],
     "poro_pc_mg_info": [vp, C.c_char_p, c_i64p, C.c_int],
     "poro_pc_mg_transfer": [vp, C.c_char_p, C.c_int, C.c_int, C.c_int, vp, vp],
@@ -187,6 +191,13 @@ class Context:
         check(self.lib.poro_timer_stop(self.h, C.byref(ms)))
         return ms.value
 
+    def dense_inverse(self, A):
+        """Gauss-Jordan inverse of a dense host matrix on the device (the coarsest AMG level's solver)."""
+        A = np.ascontiguousarray(A, dtype=np.float64)
+        inv = np.empty_like(A)
+        check(self.lib.poro_dense_inverse(self.h, A.shape[0], _ptr(A), _ptr(inv)))
+        return inv
+
     def init_dist(self, rank: int, nranks: int, unique_id: bytes):
         check(self.lib.poro_ctx_init_dist(self.h, rank, nranks, unique_id))
         self.rank, self.nranks = rank, nranks
@@ -239,6 +250,26 @@ class Mat:
 
     def mult(self, x, y):
         check(self.ctx.lib.poro_mat_mult(self.h, _ptr(x), _ptr(y)))
+
+    def to_scipy(self):
+        """Host copy of the device CSR as it is stored (explicit zeros kept)."""
+        import scipy.sparse as sp
+        r, c, z = self.info()
+        rp, ci, v = np.zeros(r + 1, np.int64), np.zeros(z, np.int32), np.zeros(z, np.float64)
+        check(self.ctx.lib.poro_mat_copy(self.h, _ptr(rp), _ptr(ci), _ptr(v)))
+        return sp.csr_matrix((v, ci, rp), shape=(r, c))
+
+    def setup_op(self, other, op: str, alpha: float = 0.0, s=None):
+        """One set-up primitive (poro_mat_setup_op): ("spgemm", B) self B, ("transpose", None) self^T, ("add_scaled", B)
+        self + alpha diag(s) B with s a device vector or None.  Returns (new Mat, SpGEMM row chunks)."""
+        h, chunks = vp(), C.c_int()
+        check(self.ctx.lib.poro_mat_setup_op(self.h, other.h if other is not None else None, op.encode(), float(alpha), _ptr(s),
+                                             C.byref(h), C.byref(chunks)))
+        m = Mat.__new__(Mat)
+        r, c, _ = (C.c_int64(), C.c_int64(), C.c_int64())
+        check(self.ctx.lib.poro_mat_info(h, C.byref(r), C.byref(c), None))
+        m.ctx, m.h, m.shape = self.ctx, h, (r.value, c.value)
+        return m, chunks.value
 
     def bench(self, mode: int, reps: int = 20) -> float:
         """Device milliseconds per launch of the SpMV in epilogue mode 0..4 (see include/poro.h)."""

@@ -445,6 +445,12 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
     bool have_next = false;
     std::unique_ptr<DistPlan> next_plan;
     const bool verbose = c.has_opt("-poro_verbose");
+    const bool keep = !dist && c.opt_i("-poro_amg_keep_setup", 0) != 0;
+    auto keep_B = [&](AmgLevel& L) {
+        L.keep_B.alloc((size_t)n * k);
+        PORO_CUDA(cudaMemcpyAsync(L.keep_B.p, B.p, (size_t)n * k * sizeof(double), cudaMemcpyDeviceToDevice, c.stream));
+        L.kept = true;
+    };
     while (true) {
         auto L = std::make_unique<AmgLevel>();
         if (have_next) L->A = std::move(Anext);
@@ -458,7 +464,9 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
         }
         levels.push_back(std::move(L));
         Lp->bs = bs;
+        Lp->k = k;
         n = Acur->nrows;
+        if (keep) keep_B(*Lp);
         const int n_gh = dist ? Lp->plan->n_ghost : 0;
         const int64_t n_glob = dist ? Lp->plan->offsets.back() : n;
         if (dist && levels.size() >= 2 && !par.smoother_only && n_glob > par.coarse_size &&
@@ -505,6 +513,7 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
                 if (off <= 1e-14 * fabs(d)) for (int j = 0; j < kk; ++j) b[(size_t)i * kk + j] = 0.0;
             });
         }
+        if (keep) keep_B(*Lp);
         if (geo_next) {
             // the same block generated at N/2 (rediscretisation = Galerkin product with the geometric transfer), the
             // near-nullspace injected at the coinciding nodes (exact for the rigid-body modes: the coarse space holds them)
@@ -556,14 +565,14 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
         if (!dist) {
             {
                 Csr AT;
-                { Tick t(c, "spgemm A*T"); csr_spgemm(c, *Acur, T, AT); }
+                { Tick t(c, "spgemm A*T"); csr_spgemm(c, *Acur, T, AT, &Lp->spgemm_chunks[0]); }
                 csr_add_scaled(c, T, AT, -omega, Lp->dinv.p, Lp->P);
             }
             { Tick t(c, "transpose P"); csr_transpose(c, Lp->P, Lp->R); }
             {
                 Csr AP;
-                { Tick t(c, "spgemm A*P"); csr_spgemm(c, *Acur, Lp->P, AP); }
-                { Tick t(c, "spgemm R*(AP)"); csr_spgemm(c, Lp->R, AP, Ac); }
+                { Tick t(c, "spgemm A*P"); csr_spgemm(c, *Acur, Lp->P, AP, &Lp->spgemm_chunks[1]); }
+                { Tick t(c, "spgemm R*(AP)"); csr_spgemm(c, Lp->R, AP, Ac, &Lp->spgemm_chunks[2]); }
             }
             // dead coarse dofs (rank-deficient aggregates): unit diagonal
             {
@@ -582,6 +591,10 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
             next_plan = std::make_unique<DistPlan>(std::move(o.coarse_plan));
         }
         Lp->n_agg = n_agg;
+        if (keep) {
+            Lp->keep_agg = std::move(agg);
+            Lp->keep_T = std::move(T);
+        }
         {
             // block structure of the transfer operators and of the coarse operator (k modes per aggregate)
             const int hint = (bs % 3 == 0 && k % 3 == 0) ? 3 : ((bs % 2 == 0 && k % 2 == 0) ? 2 : 0);

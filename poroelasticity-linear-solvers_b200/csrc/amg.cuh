@@ -34,6 +34,14 @@ struct AmgLevel {
     bool replicated = false;        // this level and everything below is gathered on every rank and cycled redundantly (Amg::tail)
     DBuf<double> ext;               // staging for vectors that are not stored extended (the caller's x on level 0)
     std::unique_ptr<MgTransfer> mg; // geometric level: the transfer to the next level replaces P and R
+    int k = 0;                      // near-nullspace modes of this level
+    int spgemm_chunks[3] = {0, 0, 0};   // row chunks of A T, A P and R (A P)
+    // `-poro_amg_keep_setup 1` (tests of the set-up): the aggregates (-1 = not aggregated), the near-nullspace as this level
+    // used it (after the Dirichlet zeroing; the coarsest level's as received) and the tentative prolongator
+    bool kept = false;
+    DBuf<int> keep_agg;
+    DBuf<double> keep_B;
+    Csr keep_T;
 };
 
 struct Amg {

@@ -957,6 +957,100 @@ int poro_pc_amg_info(poro_pc* pc, const char* name, int64_t* rows, int64_t* nnz,
     API_END
 }
 
+static Amg& amg_level_of(poro_pc* pc, const char* name, int level, const char* who) {
+    KSP* k = find_ksp(pc, name ? name : "");
+    if (!k) throw Error(std::string(who) + ": no such inner solver: " + (name ? name : ""));
+    PCAmg* a = dynamic_cast<PCAmg*>(k->pc);
+    if (!a) throw Error(std::string(who) + ": inner solver '" + name + "' has no AMG hierarchy");
+    PORO_REQUIRE(!a->amg.dist, std::string(who) + ": the hierarchy of '" + name + "' is row-partitioned");
+    PORO_REQUIRE(level >= 0 && level < (int)a->amg.levels.size(), std::string(who) + ": level " + std::to_string(level) + " out of range (" +
+                                                                   std::to_string(a->amg.levels.size()) + " levels)");
+    return a->amg;
+}
+
+int poro_pc_amg_level_info(poro_pc* pc, const char* name, int level, int64_t* out, int n, double* lmax) {
+    API_BEGIN
+    Amg& a = amg_level_of(pc, name, level, "poro_pc_amg_level_info");
+    const AmgLevel& L = *a.levels[level];
+    const bool last = level + 1 == (int)a.levels.size();
+    std::vector<int64_t> v;
+    auto dims = [&](const Csr& M) { v.push_back(M.nrows); v.push_back(M.ncols); v.push_back(M.nnz); };
+    dims(a.op(level));
+    dims(L.P);
+    dims(L.R);
+    dims(L.keep_T);
+    v.insert(v.end(), {L.bs, L.k, L.n_agg, L.mg ? 1 : 0, last ? 1 : 0, last && a.coarse_direct ? 1 : 0, L.kept ? 1 : 0,
+                       L.spgemm_chunks[0], L.spgemm_chunks[1], L.spgemm_chunks[2]});
+    for (int i = 0; i < n; ++i) out[i] = i < (int)v.size() ? v[i] : 0;
+    if (lmax) *lmax = L.lmax;
+    API_END
+}
+
+int poro_pc_amg_level_copy(poro_pc* pc, const char* name, int level, const char* what, int64_t* rowptr, int32_t* col, double* val) {
+    API_BEGIN
+    Amg& a = amg_level_of(pc, name, level, "poro_pc_amg_level_copy");
+    const AmgLevel& L = *a.levels[level];
+    const std::string w = what ? what : "";
+    const std::string at = "poro_pc_amg_level_copy('" + w + "', level " + std::to_string(level) + "): ";
+    const bool last = level + 1 == (int)a.levels.size();
+    auto csr_out = [&](const Csr& M) {
+        std::vector<int> rp, ci;
+        std::vector<double> v;
+        csr_to_host(M, rp, ci, v);
+        for (size_t i = 0; i < rp.size(); ++i) rowptr[i] = rp[i];
+        for (size_t i = 0; i < ci.size(); ++i) { col[i] = ci[i]; val[i] = v[i]; }
+    };
+    auto dev_out = [&](const void* src, size_t bytes, void* dst) {
+        PORO_CUDA(cudaStreamSynchronize(a.ctx->stream));
+        if (bytes) PORO_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost));
+    };
+    if (w == "A") { csr_out(a.op(level)); return 0; }
+    if (w == "dinv") { dev_out(L.dinv.p, (size_t)a.op(level).nrows * sizeof(double), val); return 0; }
+    if (w == "inv") {
+        PORO_REQUIRE(last && a.coarse_direct, at + "only the coarsest level of a hierarchy solved directly has an inverse");
+        dev_out(a.coarse_inv.p, a.coarse_inv.bytes(), val);
+        return 0;
+    }
+    const bool transfer = w == "P" || w == "R" || w == "T";
+    PORO_REQUIRE(transfer || w == "agg" || w == "B", at + "unknown item (A P R T agg B dinv inv)");
+    PORO_REQUIRE(!(L.mg && w != "B"), at + "the level is geometric: its transfer has no matrix and it has no aggregates");
+    PORO_REQUIRE(!(last && w != "B"), at + "the coarsest level has no transfer and no aggregates");
+    if (w == "P" || w == "R") { csr_out(w == "P" ? L.P : L.R); return 0; }
+    PORO_REQUIRE(L.kept, at + "the set-up data was not kept (set -poro_amg_keep_setup 1 before the set-up)");
+    if (w == "T") csr_out(L.keep_T);
+    else if (w == "agg") dev_out(L.keep_agg.p, L.keep_agg.bytes(), col);
+    else dev_out(L.keep_B.p, L.keep_B.bytes(), val);
+    API_END
+}
+
+int poro_mat_setup_op(poro_mat* a, poro_mat* b, const char* op, double alpha, const double* s_dev, poro_mat** out, int* chunks) {
+    API_BEGIN
+    Ctx& c = a->ctx->c;
+    const std::string o = op ? op : "";
+    PORO_REQUIRE(o == "transpose" || (b && b->ctx == a->ctx), "poro_mat_setup_op: '" + o + "' needs a second matrix of the same context");
+    Csr C;
+    int ch = 0;
+    if (o == "spgemm") csr_spgemm(c, a->raw, b->raw, C, &ch);
+    else if (o == "transpose") csr_transpose(c, a->raw, C);
+    else if (o == "add_scaled") csr_add_scaled(c, a->raw, b->raw, alpha, s_dev, C);
+    else throw Error("poro_mat_setup_op: unknown operation '" + o + "' (spgemm transpose add_scaled)");
+    PORO_CUDA(cudaStreamSynchronize(c.stream));
+    if (chunks) *chunks = ch;
+    *out = poro_mat_adopt(a->ctx, std::move(C));
+    API_END
+}
+
+int poro_dense_inverse(poro_ctx* h, int n, const double* a_host, double* inv_host) {
+    API_BEGIN
+    Ctx& c = h->c;
+    PORO_REQUIRE(n > 0, "poro_dense_inverse: n must be positive");
+    DBuf<double> A((size_t)n * n), inv;
+    PORO_CUDA(cudaMemcpy(A.p, a_host, A.bytes(), cudaMemcpyHostToDevice));
+    dense_inverse_full(c, A.p, n, inv);
+    PORO_CUDA(cudaMemcpy(inv_host, inv.p, inv.bytes(), cudaMemcpyDeviceToHost));
+    API_END
+}
+
 static Amg& mg_amg(poro_pc* pc, const char* name) {
     KSP* k = find_ksp(pc, name ? name : "");
     if (!k) throw Error(std::string("no such inner solver: ") + (name ? name : ""));

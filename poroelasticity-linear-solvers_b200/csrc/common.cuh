@@ -310,7 +310,7 @@ enum CombineOp { COMBINE_SUM = 0, COMBINE_MAX = 1 };
 // unsorted (key = row<<32 | col, val) with duplicates -> CSR with sorted unique columns. keys/vals are consumed.
 void coo_to_csr(Ctx& c, int nrows, int ncols, int64_t nent, DBuf<uint64_t>& keys, DBuf<double>& vals, Csr& out,
                 CombineOp op = COMBINE_SUM);
-void csr_spgemm(Ctx& c, const Csr& A, const Csr& B, Csr& C);            // C = A B
+void csr_spgemm(Ctx& c, const Csr& A, const Csr& B, Csr& C, int* chunks = nullptr);   // C = A B; *chunks: row chunks used
 void csr_transpose(Ctx& c, const Csr& A, Csr& At);
 // C = A[rows, cols] with maps old index -> new index (or -1 to drop); new sizes given
 void csr_extract(Ctx& c, const Csr& A, const int* row_map, const int* col_map, int new_rows, int new_cols, Csr& C);

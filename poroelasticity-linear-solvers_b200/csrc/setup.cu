@@ -139,7 +139,7 @@ void coo_to_csr(Ctx& c, int nrows, int ncols, int64_t nent, DBuf<uint64_t>& keys
 // ------------------------------------------------------------------------------------------
 // SpGEMM by expansion, chunked over rows of A
 // ------------------------------------------------------------------------------------------
-void csr_spgemm(Ctx& c, const Csr& A, const Csr& B, Csr& C) {
+void csr_spgemm(Ctx& c, const Csr& A, const Csr& B, Csr& C, int* chunks) {
     PORO_REQUIRE(A.ncols == B.nrows, "spgemm: inner dimensions differ");
     const int n = A.nrows;
     // products per row of A
@@ -205,6 +205,7 @@ void csr_spgemm(Ctx& c, const Csr& A, const Csr& B, Csr& C) {
         part_r0.push_back(r0);
         r0 = r1;
     }
+    if (chunks) *chunks = (int)parts.size();
     if (parts.size() == 1) {
         C = std::move(parts[0]);
         C.nrows = n;

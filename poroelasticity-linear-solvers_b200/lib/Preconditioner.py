@@ -92,6 +92,39 @@ class PreconditionerCC(object):
         _capi.check(self.ctx.lib.poro_pc_amg_info(self.h, name.encode(), rows, nnz, 32, C.byref(nl)))
         return [(rows[i], nnz[i]) for i in range(nl.value)]
 
+    AMG_LEVEL_KEYS = ("A_rows", "A_cols", "A_nnz", "P_rows", "P_cols", "P_nnz", "R_rows", "R_cols", "R_nnz", "T_rows", "T_cols",
+                      "T_nnz", "bs", "k", "n_agg", "geometric", "coarsest", "direct", "kept", "chunks_AT", "chunks_AP", "chunks_RAP")
+
+    def amg_level_info(self, name, level):
+        """One level of a block's AMG hierarchy (poro_pc_amg_level_info) as a dict (keys: AMG_LEVEL_KEYS and "lmax")."""
+        out, lmax = (C.c_int64 * len(self.AMG_LEVEL_KEYS))(), C.c_double()
+        _capi.check(self.ctx.lib.poro_pc_amg_level_info(self.h, name.encode(), int(level), out, len(out), C.byref(lmax)))
+        d = dict(zip(self.AMG_LEVEL_KEYS, (int(v) for v in out)))
+        d["lmax"] = lmax.value
+        return d
+
+    def amg_level(self, name, level, what):
+        """Host copy of one item of an AMG level (poro_pc_amg_level_copy): "A" "P" "R" "T" as scipy CSR (explicit zeros
+        kept), "agg" int32 (n / bs), "B" (n, k), "dinv" (n), "inv" (n, n).  "agg", "B" and "T" need -poro_amg_keep_setup 1."""
+        import scipy.sparse as sp
+        info = self.amg_level_info(name, level)
+        n = info["A_rows"]
+        rp = ci = v = None
+        if what in ("A", "P", "R", "T"):
+            r, c, z = info[what + "_rows"], info[what + "_cols"], info[what + "_nnz"]
+            rp, ci, v = np.zeros(r + 1, np.int64), np.zeros(z, np.int32), np.zeros(z, np.float64)
+        elif what == "agg":
+            ci = np.zeros(n // max(info["bs"], 1), np.int32)
+        else:
+            v = np.zeros({"B": n * info["k"], "dinv": n, "inv": n * n}.get(what, 0), np.float64)
+        _capi.check(self.ctx.lib.poro_pc_amg_level_copy(self.h, name.encode(), int(level), what.encode(), _capi._ptr(rp),
+                                                        _capi._ptr(ci), _capi._ptr(v)))
+        if rp is not None:
+            return sp.csr_matrix((v, ci, rp), shape=(r, c))
+        if what == "agg":
+            return ci
+        return v.reshape(n, -1) if what in ("B", "inv") else v
+
     FACTOR_INFO_KEYS = ("rows", "nnz_l", "nnz_u", "amalgamation_zeros", "supernodes", "levels", "max_front",
                         "perturbed_pivots", "device_bytes", "factor_flops", "factor_us", "apply_bytes")
 
