@@ -45,13 +45,17 @@ def build(block: str, N: int, overrides=None, assemble="device", ctx=None, optio
     host = None
     if assemble == "device":
         from poro_b200.generator import generate_swelling3d
-        # `-<prefix>pc_type mg` on the block: attach every coarse level N allows (halving while N stays even)
+        from poro_b200.generator import max_mg_levels
+        # under torchrun every rank generates its z-slab (the process group is initialised by `run`)
+        rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
+        # `-<prefix>pc_type mg` on the block: attach every coarse level N and the slabs allow (halving while N stays even
+        # and every rank keeps two P2 planes)
         prefixes = ("s_",) if block == "s" else ("fp_fieldsplit_0_",)
         mg_levels = 1
         if any(str(ctx.get_option("-" + p + "pc_type", "")) == "mg" for p in prefixes):
-            while N % (1 << mg_levels) == 0:
-                mg_levels += 1
-        g = generate_swelling3d(ctx, N, "diagonal", overrides=ov, mg_levels=mg_levels)
+            mg_levels = max_mg_levels(N, world)
+        g = generate_swelling3d(ctx, N, "diagonal", rank, world, overrides=ov, mg_levels=mg_levels,
+                                init_dist=getattr(ctx, "nranks", 1) != world)
         A, b, imap, par, bcs_p = g.A, g.b, g.index_set(), g.par, g.bcs_sub_pressure
         ns, nf, npp = g.layout.n_field
     else:
@@ -74,6 +78,13 @@ def run(block: str, default_N: int, argv=None):
     from poro_b200.lib.Parser import Parser, load_petsc_options
     from poro_b200.lib.Printing import parprint
     from poro_b200.lib.backend import get_context
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        import torch
+        import torch.distributed as dist
+        local = int(os.environ.get("LOCAL_RANK", "0"))
+        torch.cuda.set_device(local)
+        if not dist.is_initialized():
+            dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     ctx = get_context()
     load_petsc_options(ctx, DEFAULTS[block], is_text=True)
     parser = Parser(argv, ctx=ctx)                           # --petsc-options FILE overrides the defaults

@@ -145,7 +145,8 @@ int poro_pc_setup(poro_ctx* ctx, poro_mat* A, poro_mat* P, poro_mat* P_diff_or_n
 int poro_pc_apply(poro_pc* pc, const double* x_dev, double* y_dev);
 int poro_pc_destroy(poro_pc* pc);
 /* t_total, t_solid, t_fluid, t_press, t_alloc (lib/Preconditioner.py:252-260), then
- * per-block inner iteration totals and call counts: s, f, p, fp, diff, fp_split0, fp_split1 */
+ * per-block inner iteration totals and call counts: s, f, p, fp, diff, fp_split0, fp_split1, then the number of
+ * applications replayed from the captured CUDA graph */
 int poro_pc_stats(poro_pc* pc, double* out, int n);
 
 /* ---- outer Krylov solver -------------------------------------------------------------

@@ -469,7 +469,7 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
         if (keep) keep_B(*Lp);
         const int n_gh = dist ? Lp->plan->n_ghost : 0;
         const int64_t n_glob = dist ? Lp->plan->offsets.back() : n;
-        if (dist && levels.size() >= 2 && !par.smoother_only && n_glob > par.coarse_size &&
+        if (dist && levels.size() >= 2 && (int)levels.size() >= par.mg_levels && !par.smoother_only && n_glob > par.coarse_size &&
             n_glob <= c.opt_i("-poro_amg_replicate_below", 0)) {
             // latency-bound level: gather it once, build and cycle the rest of the hierarchy redundantly on every rank
             Tick t(c, "gathered tail hierarchy");
@@ -478,13 +478,15 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
             tail_A.block_hint = bs;
             tail = std::make_unique<Amg>();
             AmgParams tp = par;
-            tp.max_levels = std::max(1, par.max_levels - (int)levels.size() + 1);
+            tp.mg_levels = 0;                      // the gathered levels are algebraic (below the coarsest geometric one)
+            tp.max_levels = std::max(1, par.max_levels - ((int)levels.size() - std::max(par.mg_levels - 1, 0)) + 1);
             tail->setup(c, tail_A, bs, Bg.p, k, tp, nullptr);
             tail_b.alloc((size_t)n_glob);
             tail_x.alloc((size_t)n_glob);
             Lp->replicated = true;
             Lp->x.alloc((size_t)n + n_gh);
             Lp->b.alloc(n);
+            Lp->ext.alloc((size_t)n + n_gh);       // ext() of other vectors (poro_pc_mg_transfer onto this level)
             if (verbose && c.rank == 0)
                 fprintf(stderr, "    [amg] level %d: %lld global rows gathered on every rank, %d redundant levels below\n", (int)levels.size() - 1,
                         (long long)n_glob, (int)tail->levels.size());
@@ -516,13 +518,14 @@ void Amg::setup(Ctx& c, const Csr& A, int bs, const double* B_dev, int k, const 
         if (keep) keep_B(*Lp);
         if (geo_next) {
             // the same block generated at N/2 (rediscretisation = Galerkin product with the geometric transfer), the
-            // near-nullspace injected at the coinciding nodes (exact for the rigid-body modes: the coarse space holds them)
+            // near-nullspace injected at the coinciding nodes (exact for the rigid-body modes: the coarse space holds them).
+            // Row-partitioned: the coarse slab block brings its halo plan, the next level's plan
             Tick t(c, "geometric level");
             Csr Ac;
-            mg_coarse_block(c, *Acur->stencil, Ac);
+            mg_coarse_block(c, *Acur->stencil, Ac, dist ? &next_plan : nullptr);
             Ac.block_hint = bs;
             Lp->mg = std::make_unique<MgTransfer>();
-            mg_transfer_init(c, *Lp->mg, *Acur->stencil, *Ac.stencil);
+            mg_transfer_init(c, *Lp->mg, *Acur->stencil, *Ac.stencil, dist ? next_plan.get() : nullptr);
             DBuf<double> Bc;
             mg_inject(c, *Lp->mg, B.p, k, Bc);
             Anext = std::move(Ac);
@@ -746,7 +749,7 @@ void Amg::cycle(int l, const double* b, double* x) {
     if (L.mg) mg_restrict(c, *L.mg, L.r.p, Ln.b.p);
     else spmv(c, L.R, ext(l, L.r.p), Ln.b.p);                          // restriction reads the ghost residuals
     cycle(l + 1, Ln.b.p, Ln.x.p);
-    if (L.mg) mg_prolong(c, *L.mg, Ln.x.p, x, true);
+    if (L.mg) mg_prolong(c, *L.mg, ext(l + 1, Ln.x.p), x, true);      // the coarse ghosts the prolongation reads
     else spmv(c, L.P, ext(l + 1, Ln.x.p), x, SPMV_ADD, x);             // prolongation reads the ghost coarse values
     if (par.post_smooth) cheby(l, b, x, false);
 }

@@ -244,10 +244,22 @@ int poro_mat_set_coarse(poro_mat* fine, poro_mat* coarse) {
     const Csr& F = fine->raw;
     const Csr& G = coarse->raw;
     auto generated = [](const Csr& M) { return M.stencil && M.stencil->fr < 0; };
-    PORO_REQUIRE(generated(F), "poro_mat_set_coarse: the fine matrix was not generated by poro_gen_matrix on one rank");
-    PORO_REQUIRE(generated(G), "poro_mat_set_coarse: the coarse matrix was not generated by poro_gen_matrix on one rank");
+    PORO_REQUIRE(generated(F), "poro_mat_set_coarse: the fine matrix was not generated by poro_gen_matrix (whole lattices on one "
+                               "rank, or a z-slab of the cube on several)");
+    PORO_REQUIRE(generated(G), "poro_mat_set_coarse: the coarse matrix was not generated by poro_gen_matrix (whole lattices on one "
+                               "rank, or a z-slab of the cube on several)");
     const StencilData& f = *F.stencil->d;
     const StencilData& g = *G.stencil->d;
+    PORO_REQUIRE(f.slab == g.slab, "poro_mat_set_coarse: one matrix is a row-partitioned slab, the other holds whole lattices");
+    if (f.slab) {
+        // nested slabs: coarse P2 plane k is fine P2 plane 2k, so the coarse slab of fine planes [a, b) is [ceil(a/2), ceil(b/2))
+        const int64_t sf = (int64_t)(2 * f.N + 1) * (2 * f.N + 1), sg = (int64_t)(2 * g.N + 1) * (2 * g.N + 1);
+        const int64_t a = f.o0[1] / sf, b = f.o1[1] / sf, ca = g.o0[1] / sg, cb = g.o1[1] / sg;
+        PORO_REQUIRE(f.N == 2 * g.N && ca == (a + 1) / 2 && cb == (b + 1) / 2,
+                     "poro_mat_set_coarse: the slabs do not nest: fine P2 planes [" + std::to_string(a) + ", " + std::to_string(b) +
+                         ") need coarse planes [" + std::to_string((a + 1) / 2) + ", " + std::to_string((b + 1) / 2) + "), the coarse slab owns [" +
+                         std::to_string(ca) + ", " + std::to_string(cb) + ")");
+    }
     PORO_REQUIRE(f.dim == g.dim, "poro_mat_set_coarse: dim differs (fine " + std::to_string(f.dim) + ", coarse " + std::to_string(g.dim) + ")");
     PORO_REQUIRE(f.N == 2 * g.N, "poro_mat_set_coarse: N_fine must be 2 N_coarse (fine N = " + std::to_string(f.N) + ", coarse N = " +
                                      std::to_string(g.N) + ")");
@@ -420,8 +432,12 @@ int poro_fields_set(poro_ctx* h, const int64_t* is_s, int64_t ns, const int64_t*
         k = 0;
         for (int64_t g : halo_lists[t]) new_of_old[g] = (int)(n_owned + fl.hoff[t] + k++);
     }
-    fl.identity = true;
-    for (int64_t g = 0; g < n_ext; ++g) if (new_of_old[g] != (int)g) { fl.identity = false; break; }
+    fl.identity = fl.owned_identity = true;
+    for (int64_t g = 0; g < n_ext; ++g)
+        if (new_of_old[g] != (int)g) {
+            fl.identity = false;
+            if (g < n_owned) fl.owned_identity = false;
+        }
     std::vector<int> old_of_new((size_t)n_owned);
     for (int64_t g = 0; g < n_owned; ++g) old_of_new[new_of_old[g]] = (int)g;
     fl.new_of_old.alloc((size_t)n_ext);
@@ -481,6 +497,14 @@ static bool stencil_layout_matches(const Fields& fl, const StencilOp& s) {
     return true;
 }
 
+// the owned rows of the solver's fields are the generator's owned rows in the generator's order (halos may be reordered)
+static bool slab_layout_matches(const Fields& fl, const StencilOp& s) {
+    if (!fl.owned_identity || !s.d->slab) return false;
+    for (int t = 0; t < 3; ++t)
+        if (fl.off[t] != s.d->row0[t] || fl.n[t] != s.d->row0[t + 1] - s.d->row0[t]) return false;
+    return true;
+}
+
 // columns: list of (field) pieces in order; rows: contiguous permuted range [r0, r1)
 static std::unique_ptr<MatOp> extract_block(poro_ctx* h, const Csr& Mp, int64_t r0, int64_t r1, std::vector<int> col_fields) {
     Ctx& c = h->c;
@@ -517,6 +541,11 @@ static std::unique_ptr<MatOp> extract_block(poro_ctx* h, const Csr& Mp, int64_t 
                 op->M.stencil = std::make_shared<StencilOp>(StencilOp{Mp.stencil->d, fr, col_fields[0]});
                 break;
             }
+    }
+    // a diagonal field block of a row-partitioned slab keeps its descriptor for `-<prefix>pc_type mg` (never applied from it)
+    if (Mp.stencil && Mp.stencil->fr < 0 && c.nranks > 1 && col_fields.size() == 1 && slab_layout_matches(fl, *Mp.stencil)) {
+        const int fr = col_fields[0];
+        if (r0 == fl.off[fr] && r1 == fl.off[fr] + fl.n[fr]) op->M.stencil = std::make_shared<StencilOp>(StencilOp{Mp.stencil->d, fr, fr});
     }
     return op;
 }
@@ -558,9 +587,6 @@ static std::unique_ptr<KSP> make_inner(poro_ctx* h, MatOp* op, const std::string
     std::string pt = c.opt("-" + prefix + "pc_type", pc_type);
     if (pt == "fieldsplit") pt = "amg";
     const Csr* src = &op->mat();
-    if (pt == "mg" && c.nranks > 1)
-        throw Error("-" + prefix + "pc_type mg: geometric multigrid runs on one rank, this block is row-partitioned over " +
-                    std::to_string(c.nranks) + " ranks");
     const bool amg_type = pt == "hypre" || pt == "amg" || pt == "gamg" || pt == "ml" || pt == "chebyshev" || pt == "mg";
     // row-partitioned runs: hierarchies are distributed (global Galerkin coarse levels, distamg.cu) whenever the block has
     // ONE halo plan; the decision uses global sizes so that every rank takes the same (collective) path
@@ -840,6 +866,7 @@ int poro_pc_stats(poro_pc* pc, double* out, int n) {
     add(cc.ksp_s.get()); add(cc.ksp_f.get()); add(cc.ksp_p.get()); add(cc.ksp_fp.get()); add(cc.ksp_diff.get());
     add(cc.schur ? cc.schur->k0.get() : nullptr);
     add(cc.schur ? cc.schur->k1.get() : nullptr);
+    v.push_back((double)cc.graph_replays);
     for (int i = 0; i < n; ++i) out[i] = i < (int)v.size() ? v[i] : 0.0;
     API_END
 }
@@ -876,7 +903,7 @@ int poro_pc_block_bytes(poro_pc* pc, const char* name, int64_t* bytes, int* form
     MatOp* m = find_block(pc, name);
     if (!m) throw Error(std::string("no such block: ") + name);
     const Csr& B = m->mat();
-    if (B.stencil && B.stencil->fr >= 0) {
+    if (stencil_runs(B)) {
         *bytes = stencil_bytes(*B.stencil);
         *format = 4;
         return 0;
@@ -1070,7 +1097,7 @@ int poro_pc_mg_info(poro_pc* pc, const char* name, int64_t* out, int n) {
         const bool st = A.stencil && A.stencil->fr >= 0;
         v.push_back(st ? A.stencil->d->N : -1);
         v.push_back(A.nrows);
-        v.push_back(st ? 4 : 0);
+        v.push_back(stencil_runs(A) ? 4 : 0);
     }
     v.push_back((int64_t)a.levels.size() - geo);
     for (int i = 0; i < n; ++i) out[i] = i < (int)v.size() ? v[i] : 0;
@@ -1086,7 +1113,7 @@ int poro_pc_mg_transfer(poro_pc* pc, const char* name, int level, int dir, int m
     PORO_REQUIRE(mode == 0 || mode == 1, "poro_pc_mg_transfer: mode is 0 (set) or 1 (add)");
     PORO_REQUIRE(dir == 0 || mode == 0, "poro_pc_mg_transfer: restriction has mode 0 only");
     Ctx& c = pc->ctx->c;
-    if (dir == 0) mg_prolong(c, *a.levels[level]->mg, x, y, mode == 1);
+    if (dir == 0) mg_prolong(c, *a.levels[level]->mg, a.ext(level + 1, x), y, mode == 1);   // row-partitioned: coarse ghosts of x
     else mg_restrict(c, *a.levels[level]->mg, x, y);
     API_END
 }

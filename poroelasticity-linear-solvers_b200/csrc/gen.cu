@@ -233,7 +233,9 @@ int poro_gen_matrix(poro_ctx* h, int dim, int N, const poro_gen_table* tables, c
         PORO_REQUIRE(herr == 0, "generator: a stencil entry falls outside the owned and ghost node ranges of the layout");
         csr_choose_lanes(A);
         // single rank, whole lattices owned: keep the tables next to the CSR so that products run from them (stencil.cu).
-        // Row-partitioned slabs order their ghost columns differently from the field blocks extracted later: assembled only.
+        // Row-partitioned slabs order their ghost columns differently from the field blocks extracted later: their products
+        // stay assembled, the descriptor only carries the geometry of `-<prefix>pc_type mg` (slab = true).
+        const bool slab = c.nranks > 1 && dim == 3;
         bool whole = c.nranks == 1;
         for (int k = 0; k < 2; ++k)
             whole = whole && g.o0[k] == 0 && g.o1[k] == porogen::lattice_nodes(k + 1, N, dim) && g.gl0[k] == g.gl1[k] && g.gu0[k] == g.gu1[k];
@@ -250,9 +252,14 @@ int poro_gen_matrix(poro_ctx* h, int dim, int N, const poro_gen_table* tables, c
                 whole = bnd;
             }
         }
-        if (whole) {
+        if (whole || slab) {
             auto d = std::make_shared<StencilData>();
             d->dim = dim; d->N = N;
+            d->slab = !whole;
+            for (int k = 0; k < 2; ++k) {
+                d->o0[k] = g.o0[k]; d->o1[k] = g.o1[k]; d->gl0[k] = g.gl0[k]; d->gl1[k] = g.gl1[k]; d->gu0[k] = g.gu0[k]; d->gu1[k] = g.gu1[k];
+            }
+            for (int f = 0; f < 3; ++f) { d->off_gl[f] = g.off_gl[f]; d->off_gu[f] = g.off_gu[f]; }
             for (int b = 0; b < 9; ++b) {
                 d->t[b] = T.t[b]; d->present[b] = T.present[b]; d->diag_only[b] = diag_only[b]; d->table_bytes[b] = table_bytes[b];
                 d->cls[b] = std::move(d_cls[b]); d->off[b] = std::move(d_off[b]); d->val[b] = std::move(d_val[b]);
@@ -260,7 +267,7 @@ int poro_gen_matrix(poro_ctx* h, int dim, int N, const poro_gen_table* tables, c
             d->bc = std::move(d_bc);
             for (int f = 0; f < 4; ++f) d->row0[f] = g.row0[f];
             for (int f = 0; f < 3; ++f) { d->bdim[f] = g.bdim[f]; d->kind[f] = g.kind[f]; }
-            stencil_build_warps(c, *d);
+            if (!d->slab) stencil_build_warps(c, *d);
             A.stencil = std::make_shared<StencilOp>();
             A.stencil->d = std::move(d);
         }

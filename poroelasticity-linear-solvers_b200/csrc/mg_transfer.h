@@ -113,4 +113,27 @@ inline Table restrict_table(int kind, int dim) {
     return T;
 }
 
+// planes [lo, hi) of the target lattice that the rows of the planes [a, b) of the source lattice reach along axis dim - 1
+// (the slab axis of a row partition): prolongation rows of fine planes Z reach coarse planes S (Z / M) + d, restriction
+// rows of coarse planes Y fine planes 2 Y + d (planes outside [0, L_to) skipped, as the restriction kernel skips them).
+// lo = hi = a when no row has an entry.
+inline void plane_reach(const Table& T, int dim, bool prolong, int kind, int64_t a, int64_t b, int64_t L_to, int64_t& lo, int64_t& hi) {
+    const int M = fine_per_cell(kind), S = coarse_per_cell(kind), R = prolong ? M : S;
+    int stride = 1;
+    for (int m = 0; m < dim - 1; ++m) stride *= R;
+    lo = a; hi = a;
+    bool any = false;
+    for (int64_t Z = a; Z < b; ++Z)
+        for (int cls = 0; cls < T.ncls; ++cls) {
+            if ((cls / stride) % R != Z % R) continue;
+            for (int p = T.ptr[cls]; p < T.ptr[cls + 1]; ++p) {
+                const int64_t t = (prolong ? S * (Z / M) : 2 * Z) + T.e[p].d[dim - 1];
+                if (t < 0 || t >= L_to) continue;
+                lo = any ? std::min(lo, t) : t;
+                hi = any ? std::max(hi, t + 1) : t + 1;
+                any = true;
+            }
+        }
+}
+
 }  // namespace poromg

@@ -148,10 +148,11 @@ std::unique_ptr<PC> make_pc(Ctx& c, const std::string& pc_type, const Csr& A, in
     int mg_levels = 0;
     if (mg) {
         const std::string key = "-" + prefix + "pc_type mg";
-        if (plan || c.nranks > 1) throw Error(key + ": geometric multigrid runs on one rank only");
         if (!A.stencil || A.stencil->fr < 0 || A.stencil->fc != A.stencil->fr)
             throw Error(key + " needs a single generated field block; this block has no class-stencil descriptor (uploaded "
                         "through poro_mat_create_csr, permuted, cut across several fields, or a Schur complement)");
+        if (c.nranks > 1 && !(plan && A.stencil->d->slab))
+            throw Error(key + ": a row-partitioned block runs the distributed hierarchy on its generated slabs (-poro_amg_distributed 1)");
         const int attached = mg_attached_levels(*A.stencil);
         if (attached == 0)
             throw Error(key + ": the generated matrix has no coarse levels attached (poro_mat_set_coarse, or mg_levels > 1 in "
@@ -980,6 +981,7 @@ void PCBlockCC::apply(const double* x, double* y) {
     }
     vec_copy(c, g_in.p, x, n);
     PORO_CUDA(cudaGraphLaunch(gexec, c.stream));
+    ++graph_replays;
     vec_copy(c, y, g_out.p, n);
     c.launches += g_launches;
     if (!fresh)

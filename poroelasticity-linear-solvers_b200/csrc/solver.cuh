@@ -16,6 +16,7 @@ struct Fields {
     DBuf<int> new_of_old;   // extended raw index -> extended permuted index
     DBuf<int> old_of_new;   // owned permuted index -> owned raw index
     bool identity = false;
+    bool owned_identity = false;    // the owned entries keep their raw order (identity may still permute the halo)
     int block_dim = 0;
     int coord_dim = 0;
     std::vector<double> coords_s, coords_p;   // host copies, permuted order
@@ -228,6 +229,7 @@ struct PCBlockCC : PC {
     cudaGraphExec_t gexec = nullptr;
     DBuf<double> g_in, g_out;
     int64_t g_launches = 0;
+    int64_t graph_replays = 0;      // applications that ran as the captured graph (poro_pc_stats)
     std::vector<KSP*> g_ksps;
     // 2-way `diagonal` splitting: P_fp,s is structurally empty, so the solid solve and the fluid-pressure solve are independent.
     // Inside the captured graph they are forked onto two streams (two parallel branches of the graph): the latency-bound

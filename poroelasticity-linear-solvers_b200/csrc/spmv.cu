@@ -201,7 +201,7 @@ template <int MODE>
 static int launch_spmv(Ctx& c, const Csr& A, const double* x, double* y, const Epilogue& ep, double* dot_partial) {
     if (A.nrows == 0) return 0;
     // a generated block along whole fields: apply its class tables (stencil.cu) instead of streaming the assembled matrix
-    if (A.stencil && A.stencil->fr >= 0) return stencil_launch<MODE>(c, *A.stencil, x, y, ep, dot_partial);
+    if (stencil_runs(A)) return stencil_launch<MODE>(c, *A.stencil, x, y, ep, dot_partial);
     if (A.block_hint > 1 && A.bsr_state < 0) try_bsr(c, A);
     if (A.bsr_state == 1) return bsr_launch<MODE>(c, *A.bsr, x, y, ep, dot_partial);
     if (A.nblk < 0) build_row_blocks(c, A);
@@ -239,7 +239,7 @@ static int launch_spmv(Ctx& c, const Csr& A, const double* x, double* y, const E
 void spmv_kernel_info(Ctx& c, const Csr& A, int64_t* v) {
     std::fill(v, v + kSpmvInfoFields, (int64_t)0);
     v[7] = -1;
-    if (A.stencil && A.stencil->fr >= 0) { v[0] = 4; return; }
+    if (stencil_runs(A)) { v[0] = 4; return; }
     if (A.nrows > 0 && csr_ensure_bsr(c, A)) {
         const Bsr& B = *A.bsr;
         const bool plain = !B.t_ok;
@@ -301,7 +301,7 @@ __global__ void k_sum_to(const double* __restrict__ partial, int n, double* __re
 void spmv_dot(Ctx& c, const Csr& A, const double* p, double* w, double* d_dot) {
     Epilogue ep{};
     ep.mode = 4;
-    const bool st = A.stencil && A.stencil->fr >= 0;
+    const bool st = stencil_runs(A);
     if (!st && A.nblk < 0) build_row_blocks(c, A);
     const int L = A.lanes ? A.lanes : 32;
     const int64_t grid = st ? stencil_grid(*A.stencil)

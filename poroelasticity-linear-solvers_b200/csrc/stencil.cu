@@ -196,6 +196,7 @@ int stencil_grid(const StencilOp& s) { return ceil_div((int64_t)s.d->nwarps[s.d-
 
 template <int MODE>
 int stencil_launch(Ctx& c, const StencilOp& s, const double* x, double* y, const Epilogue& ep, double* dot_partial) {
+    PORO_REQUIRE(!s.d->slab, "k_stencil: a row-partitioned slab has ghost columns and is applied assembled");
     const StencilArgs a = stencil_args(s);
     const int grid = stencil_grid(s);
     if (grid == 0) return 0;

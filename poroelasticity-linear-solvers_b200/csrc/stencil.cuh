@@ -13,9 +13,15 @@ namespace poro {
 
 struct Epilogue;
 
-// everything one generated matrix was built from (single rank: every node of the lattices is owned, no ghosts)
+// everything one generated matrix was built from.  A whole-lattice matrix (one rank, no ghosts) is applied from it; a
+// row-partitioned slab (`slab`) keeps it for the geometry of its geometric transfers (mg.cuh) and stays assembled.
 struct StencilData {
     int dim = 0, N = 0;
+    // slab: per lattice (index kind - 1) the owned node range and the ghost node ranges of the lower / upper neighbour, and
+    // per field the first local column of its lower / upper ghosts (columns [owned s f p | lower s f p | upper s f p])
+    bool slab = false;
+    int64_t o0[2] = {0, 0}, o1[2] = {0, 0}, gl0[2] = {0, 0}, gl1[2] = {0, 0}, gu0[2] = {0, 0}, gu1[2] = {0, 0};
+    int64_t off_gl[3] = {0, 0, 0}, off_gu[3] = {0, 0, 0};
     porogen::BlockTable t[9];        // block (fr, fc) at fr * 3 + fc; device pointers into the buffers below
     int present[9] = {0};
     int diag_only[9] = {0};          // every entry of the table is a diagonal block (mass couplings M (x) I)
@@ -42,6 +48,9 @@ struct StencilOp {
     std::shared_ptr<StencilData> d;
     int fr = -1, fc = -1;
 };
+
+// products of A run from the class tables: a field block of a whole-lattice descriptor
+inline bool stencil_runs(const Csr& A) { return A.stencil && A.stencil->fr >= 0 && !A.stencil->d->slab; }
 
 // builds the per-lattice warp descriptors of `d` (host work, once per generated matrix)
 void stencil_build_warps(Ctx& c, StencilData& d);

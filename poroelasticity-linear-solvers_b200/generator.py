@@ -41,12 +41,14 @@ class SlabLayout:
     owned: list = field(default_factory=list)
     ghost_lo: list = field(default_factory=list)
     ghost_up: list = field(default_factory=list)
+    # owned P2 planes [a, b); default: the even split of slab_ranges (a coarse level takes them from its fine level)
+    p2_planes: tuple | None = None
 
     def __post_init__(self):
         d, N = self.dim, self.N
         assert d == 3, "slab layout is implemented for the structured cube"
         L2, L1 = 2 * N + 1, N + 1
-        a, b = slab_ranges(L2, self.world)[self.rank]
+        a, b = self.p2_planes if self.p2_planes is not None else slab_ranges(L2, self.world)[self.rank]
         assert b - a >= 2, "a z-slab needs at least two P2 planes"
         pa, pb = (a + 1) // 2, (b + 1) // 2                       # owned P1 planes: 2 zp in [a, b)
         lo, up = self.rank > 0, self.rank < self.world - 1
@@ -77,6 +79,13 @@ class SlabLayout:
         self.kind, self.bdim = kind, bdim
         self.n2, self.n1 = L2 ** d, L1 ** d
         self.n_global = 2 * d * self.n2 + self.n1
+
+    def coarsen(self) -> "SlabLayout":
+        """This rank's slab of the mesh at N/2 nested in this one: coarse P2 plane k is fine P2 plane 2k, so the coarse slab
+        owns the coarse planes [ceil(a/2), ceil(b/2)).  Ghosts, index sets and halo plan follow by the usual rules."""
+        assert self.N % 2 == 0, "the mesh at N/2 needs an even N"
+        a, b = self.planes2
+        return SlabLayout(self.dim, self.N // 2, self.rank, self.world, p2_planes=((a + 1) // 2, (b + 1) // 2))
 
     # ---- the arrays the C ABI wants ---------------------------------------------------------------------
     def layout_array(self) -> np.ndarray:
@@ -253,10 +262,31 @@ class WholeLayout:
 def _check_mg_levels(N: int, mg_levels: int, world: int = 1):
     if mg_levels < 1:
         raise ValueError("mg_levels must be at least 1, got %d" % mg_levels)
-    if mg_levels > 1 and world != 1:
-        raise ValueError("geometric coarse levels (mg_levels > 1) are generated on one rank only, not on %d" % world)
     if N % (1 << (mg_levels - 1)):
         raise ValueError("N = %d is not divisible by 2^(mg_levels - 1) = %d" % (N, 1 << (mg_levels - 1)))
+    if world > 1 and mg_levels > 1:
+        # every rank's slab must keep the two P2 planes a slab needs on every level
+        L2 = 2 * N + 1
+        for rank, (a, b) in enumerate(slab_ranges(L2, world)):
+            if b - a < 2:
+                raise ValueError("rank %d owns %d P2 plane(s) of the mesh at N = %d: a slab needs at least 2" % (rank, b - a, N))
+            for lev in range(1, mg_levels):
+                a, b = (a + 1) // 2, (b + 1) // 2
+                if b - a < 2:
+                    raise ValueError("mg_levels = %d: on level %d (N = %d) rank %d would own %d P2 plane(s) of %d ranks' slabs; a "
+                                     "slab needs at least 2 (use fewer levels or fewer ranks)" % (mg_levels, lev, N >> lev, rank, b - a, world))
+
+
+def max_mg_levels(N: int, world: int = 1) -> int:
+    """The most geometric levels N allows: halving while N stays even and, on `world` ranks, every slab keeps 2 P2 planes."""
+    lev = 1
+    while N % (1 << lev) == 0:
+        try:
+            _check_mg_levels(N, lev + 1, world)
+        except ValueError:
+            break
+        lev += 1
+    return lev
 
 
 def _swelling_operators(ctx, dim: int, N: int, pc_type: str, overrides, layout, p2_range=None, p1_range=None):
@@ -275,13 +305,19 @@ def _swelling_operators(ctx, dim: int, N: int, pc_type: str, overrides, layout, 
     return A, P, Pd, gen, par, loads
 
 
-def _attach_coarse_levels(ctx, dim: int, N: int, pc_type: str, overrides, mg_levels: int, ops):
+def _attach_coarse_levels(ctx, dim: int, N: int, pc_type: str, overrides, mg_levels: int, ops, layout=None):
     """Generates A, P, P_diff at N/2, N/4, ... (mg_levels - 1 levels) and links each fine matrix of `ops` to its coarse
-    chain (poro_mat_set_coarse).  The fine matrices keep the coarse ones alive; the coarse handles are released."""
+    chain (poro_mat_set_coarse).  With a SlabLayout every level is this rank's slab nested in the one above
+    (SlabLayout.coarsen).  The fine matrices keep the coarse ones alive; the coarse handles are released."""
     chains = [[m] for m in ops]
     for lev in range(1, mg_levels):
         Nc = N >> lev
-        A, P, Pd, _, _, _ = _swelling_operators(ctx, dim, Nc, pc_type, overrides, WholeLayout(dim, Nc))
+        if isinstance(layout, SlabLayout):
+            layout = layout.coarsen()
+            A, P, Pd, _, _, _ = _swelling_operators(ctx, dim, Nc, pc_type, overrides, layout, p2_range=layout.owned[1],
+                                                    p1_range=layout.owned[0])
+        else:
+            A, P, Pd, _, _, _ = _swelling_operators(ctx, dim, Nc, pc_type, overrides, WholeLayout(dim, Nc))
         for ch, m in zip(chains, (A, P, Pd)):
             ch.append(m)
     for ch in chains:
@@ -316,7 +352,8 @@ def generate_swelling2d(ctx, N: int, pc_type: str = "diagonal", overrides: dict 
 def generate_swelling3d(ctx, N: int, pc_type: str = "diagonal", rank: int = 0, world: int = 1, overrides: dict | None = None,
                         init_dist: bool = True, mg_levels: int = 1) -> GeneratedSystem:
     """swelling-3d.py on the unit cube (x 1e-2) with N cells per side: this rank's slab, generated on the device.
-    mg_levels > 1 (one rank) also generates the operators at N/2, N/4, ... and links them as geometric levels."""
+    mg_levels > 1 also generates the operators at N/2, N/4, ... (this rank's nested slab of each) and links them as
+    geometric levels."""
     from hostfem.stencil import swelling_generator      # element matrices of ONE macro cell + loads (FEniCS stand-in)
     _check_mg_levels(N, mg_levels, world)
     gen, par, loads = swelling_generator(3, N, overrides)
@@ -340,7 +377,7 @@ def generate_swelling3d(ctx, N: int, pc_type: str = "diagonal", rank: int = 0, w
     Pd = None
     if "3-way" in pc_type:
         Pd = generate_matrix(ctx, gen, lay, "P_diff", pc_type, np.concatenate([bc_s, bc_f, bc_p]))
-    _attach_coarse_levels(ctx, 3, N, pc_type, overrides, mg_levels, (A, P, Pd))
+    _attach_coarse_levels(ctx, 3, N, pc_type, overrides, mg_levels, (A, P, Pd), lay)
     t = par["t0"] + par["dt"]
     b = gen.rhs(t, **loads)[lay.owned_global()]
     is_s, is_f, is_p = lay.index_sets()

@@ -59,13 +59,14 @@ class PreconditionerCC(object):
         _capi.check(self.ctx.lib.poro_pc_apply(self.h, _capi._ptr(_tensor(x)), _capi._ptr(_tensor(y))))
 
     def stats(self):
-        out = (C.c_double * 19)()
-        _capi.check(self.ctx.lib.poro_pc_stats(self.h, out, 19))
+        out = (C.c_double * 20)()
+        _capi.check(self.ctx.lib.poro_pc_stats(self.h, out, 20))
         v = list(out)
         keys = ["s", "f", "p", "fp", "diff", "fp_split0", "fp_split1"]
         d = dict(t_total=v[0], t_solid=v[1], t_fluid=v[2], t_press=v[3], t_alloc=v[4])
         for i, k in enumerate(keys):
             d["its_" + k], d["calls_" + k] = int(v[5 + 2 * i]), int(v[6 + 2 * i])
+        d["graph_replays"] = int(v[19])
         return d
 
     def block_info(self, name):
