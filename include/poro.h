@@ -194,7 +194,8 @@ int poro_pc_block_mult(poro_pc* pc, const char* name, int mode, const double* x,
                        double* xv, const double* dinv, double c1, double c2, double* dot);
 /* copy a block to host CSR arrays sized from poro_pc_block_info (tests: createSubMatrix parity) */
 int poro_pc_block_copy(poro_pc* pc, const char* name, int64_t* rowptr, int32_t* col, double* val);
-/* one application of the inner solver of a block: "s","f","p","fp","diff" (z = K \ r) */
+/* one application of the inner solver of a block: "s","f","p","fp","diff", or a split of the fp fieldsplit "fp0","fp1"
+ * (z = K \ r) */
 int poro_pc_inner_solve(poro_pc* pc, const char* name, const double* r_dev, double* z_dev);
 /* iterations / reason / residual norm of the last application of an inner solver ("s","f","p","fp","diff","fp0","fp1"):
  * what `ksp.getIterationNumber()` reports in the single-block drivers (solid.py:177-180, fluid-pressure.py:133-136) */
@@ -219,6 +220,11 @@ int poro_pc_amg_level_copy(poro_pc* pc, const char* name, int level, const char*
  * largest front, perturbed pivots, device bytes held after set-up, flops of the numeric factorisation, its device time
  * in microseconds, algorithmic bytes of one application without refinement.  Fails for a block that is not a sparse LU. */
 int poro_pc_factor_info(poro_pc* pc, const char* name, int64_t* out, int n);
+/* incomplete factorisation of an inner PC ("s","f","p","fp","diff","fp0","fp1"; -<prefix>pc_type ilu or bjacobi, ILU(0) in
+ * natural order on the stored pattern).  out[0..n) receives, in this order: rows, nnz(L) (strictly lower), nnz(U) (strictly
+ * upper), levels of the lower and of the upper triangular solve, the smallest |u_ii|, device bytes held after set-up,
+ * algorithmic bytes of one application.  Fails for an inner PC that is not ILU / bjacobi. */
+int poro_pc_ilu_info(poro_pc* pc, const char* name, double* out, int n);
 /* geometric multigrid of a block's inner PC (`-<prefix>pc_type mg`).  out[0..n) receives the number G of geometric levels
  * (the finest included), then per geometric level N, rows and the launch format of its operator (4 = stencil), then the
  * number of algebraic levels below.  Fails for an inner PC that is not `mg`. */

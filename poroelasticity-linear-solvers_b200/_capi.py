@@ -75,6 +75,7 @@ SIGNATURES = {
     "poro_pc_amg_level_info": [vp, C.c_char_p, C.c_int, c_i64p, C.c_int, c_f64p],
     "poro_pc_amg_level_copy": [vp, C.c_char_p, C.c_int, C.c_char_p, vp, vp, vp],
     "poro_pc_factor_info": [vp, C.c_char_p, c_i64p, C.c_int],
+    "poro_pc_ilu_info": [vp, C.c_char_p, c_f64p, C.c_int],
     "poro_pc_mg_info": [vp, C.c_char_p, c_i64p, C.c_int],
     "poro_pc_mg_transfer": [vp, C.c_char_p, C.c_int, C.c_int, C.c_int, vp, vp],
     "poro_pc_mg_bytes": [vp, C.c_char_p, C.c_int, c_i64p],

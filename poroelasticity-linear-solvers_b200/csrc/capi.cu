@@ -1,6 +1,7 @@
 // capi.cu -- the extern "C" boundary (include/poro.h): object lifetimes, field permutation,
 // block extraction and the wiring of inner solvers from the PETSc-style options database.
 #include "../../include/poro.h"
+#include "ilu.cuh"
 #include "solver.cuh"
 #include <algorithm>
 #include <cmath>
@@ -718,6 +719,12 @@ int poro_pc_setup(poro_ctx* h, poro_mat* A, poro_mat* P, poro_mat* P_diff, const
             }
             auto sch = std::make_unique<PCSchur>();
             sch->ctx = &c;
+            // the exact big block always runs the full Schur factorisation
+            const std::string fs_type = fp_exact_big ? "schur" : c.opt("-fp_pc_fieldsplit_type", "schur");
+            if (fs_type == "additive") sch->type = FS_ADDITIVE;
+            else if (fs_type == "multiplicative") sch->type = FS_MULTIPLICATIVE;
+            else if (fs_type != "schur")
+                throw Error("-fp_pc_fieldsplit_type " + fs_type + " is not supported (schur, additive or multiplicative; two splits)");
             std::string order = c.opt("-fp_pc_fieldsplit_order", fp_exact_big ? "fp" : "pf");   // "pf" = reference (Preconditioner.py:113-114)
             sch->p_first = order != "fp";
             std::string fact = c.opt("-fp_pc_fieldsplit_schur_fact_type", fp_exact_big ? "full" : "lower");
@@ -732,85 +739,94 @@ int poro_pc_setup(poro_ctx* h, poro_mat* A, poro_mat* P, poro_mat* P_diff, const
             sch->A10 = extract_block(h, *Pp, fl.off[t1], fl.off[t1] + fl.n[t1], {t0});
             sch->A11 = extract_block(h, *Pp, fl.off[t1], fl.off[t1] + fl.n[t1], {t1});
             (t0 == 1 ? sch->A00 : sch->A11)->M.block_hint = bs_v;
-            // selfp: S = A11 - A10 diag(A00)^-1 A01
-            // cc (extension): the diagonal is the lumped mass + drag part of the velocity block, mass_scale * |diag(A_fs)| of
-            // the SYSTEM matrix (A_fs = -(phi^2 / (k_f dt)) M_v with the rows of fluid Dirichlet dofs zeroed, which then get 1),
-            // and the viscous limit visc_scale * P_pp is added in the application (PCSchur::solve1); oracle: SchurLowerCC
-            const std::string sprec = c.opt("-fp_pc_fieldsplit_schur_precondition", "selfp");
-            PORO_REQUIRE(sprec == "selfp" || sprec == "cc", "-fp_pc_fieldsplit_schur_precondition must be selfp or cc");
-            DBuf<double> d_mass;
-            if (sprec == "cc") {
-                PORO_REQUIRE(!sch->p_first && pc_type == "diagonal", "schur_precondition cc needs pc type 'diagonal' and -fp_pc_fieldsplit_order fp");
-                PORO_REQUIRE(A != nullptr && c.has_opt("-fp_pc_fieldsplit_schur_cc_mass_scale") && c.has_opt("-fp_pc_fieldsplit_schur_cc_visc_scale"),
-                             "schur_precondition cc needs A and the -fp_pc_fieldsplit_schur_cc_mass_scale / _visc_scale options (lib/Preconditioner.py sets them)");
-                PORO_REQUIRE(ns == nf, "schur_precondition cc expects the displacement and velocity fields on the same nodes");
-                const double ms = c.opt_d("-fp_pc_fieldsplit_schur_cc_mass_scale", 0.0);
-                sch->visc_scale = c.opt_d("-fp_pc_fieldsplit_schur_cc_visc_scale", 0.0);
-                PORO_REQUIRE(ms > 0.0 && sch->visc_scale > 0.0, "schur_precondition cc: the two scales must be positive");
-                Csr Aperm;
-                const Csr* Ap = &A->raw;
-                if (!fl.identity) { permute_matrix(h, A->raw, Aperm); Ap = &Aperm; }
-                auto Afs = extract_block(h, *Ap, of, of + nf, {0});
-                d_mass.alloc((size_t)nf);
-                csr_diag(c, Afs->M, d_mass.p);
-                vec_abs_scale(c, d_mass.p, ms, nf);
-                PORO_CUDA(cudaStreamSynchronize(c.stream));
-            }
-            DistPlan* plan0 = nullptr;
-            DistPlan* plan1 = nullptr;
-            if (c.nranks > 1 && c.opt_i("-poro_amg_distributed", 1)) { plan0 = sch->A00->plan_for_amg(); plan1 = sch->A11->plan_for_amg(); }
-            if (plan0 && plan1) {
-                // row-partitioned: exact complement of the owned rows -- the A01 rows and the diagonal of the ghost dofs of split 0
-                // arrive by one sparse-row and one vector exchange; S gets its own (wider) halo plan
-                sch->S = std::make_unique<MatOp>();
-                sch->S->ctx = &c;
-                sch->S->dplan = std::make_unique<DistPlan>();
-                dist_selfp_schur(c, *plan0, *plan1, sch->A00->mat(), sch->A01->mat(), sch->A10->mat(), sch->A11->mat(), sch->S->M,
-                                 *sch->S->dplan, d_mass.p);
-                sch->S->n_owned_cols = sch->n1;
-            } else
-            // single rank (or -poro_amg_distributed 0): from the local (owned) parts
-            {
-                Csr a00, a01, a10, a11;
-                local_square(c, *sch->A00, a00);
-                auto owned_cols = [&](const MatOp& m, int ncols_owned, Csr& o) {
-                    if (m.M.ncols == ncols_owned) { csr_copy(c, m.M, o); PORO_CUDA(cudaStreamSynchronize(c.stream)); return; }
-                    std::vector<int> rmap((size_t)m.M.nrows), cmap((size_t)m.M.ncols, -1);
-                    for (int i = 0; i < m.M.nrows; ++i) rmap[i] = i;
-                    for (int i = 0; i < ncols_owned; ++i) cmap[i] = i;
-                    DBuf<int> d_r(rmap.size()), d_c(cmap.size());
-                    PORO_CUDA(cudaMemcpy(d_r.p, rmap.data(), rmap.size() * 4, cudaMemcpyHostToDevice));
-                    PORO_CUDA(cudaMemcpy(d_c.p, cmap.data(), cmap.size() * 4, cudaMemcpyHostToDevice));
-                    csr_extract(c, m.M, d_r.p, d_c.p, m.M.nrows, ncols_owned, o);
-                };
-                owned_cols(*sch->A01, (int)sch->n1, a01);
-                owned_cols(*sch->A10, (int)sch->n0, a10);
-                owned_cols(*sch->A11, (int)sch->n1, a11);
-                DBuf<double> dinv((size_t)sch->n0);
-                if (d_mass.p) PORO_CUDA(cudaMemcpy(dinv.p, d_mass.p, (size_t)sch->n0 * 8, cudaMemcpyDeviceToDevice));
-                else csr_diag(c, a00, dinv.p);
-                std::vector<double> hd((size_t)sch->n0);
-                PORO_CUDA(cudaMemcpy(hd.data(), dinv.p, hd.size() * 8, cudaMemcpyDeviceToHost));
-                for (auto& v : hd) v = v != 0.0 ? 1.0 / v : 1.0;
-                PORO_CUDA(cudaMemcpy(dinv.p, hd.data(), hd.size() * 8, cudaMemcpyHostToDevice));
-                csr_scale_cols(c, a10, dinv.p);                      // A10 diag(A00)^-1
-                Csr prod;
-                csr_spgemm(c, a10, a01, prod);
-                sch->S = std::make_unique<MatOp>();
-                sch->S->ctx = &c;
-                csr_add_scaled(c, a11, prod, -1.0, nullptr, sch->S->M);
-            }
-            const int bs0 = t0 == 1 ? bs_v : 1, bs1 = t1 == 1 ? bs_v : 1;
-            const char* sub_pc = fp_exact_big ? "lu" : "amg";
-            sch->k0 = make_inner(h, sch->A00.get(), "preonly", sub_pc, "fp_fieldsplit_0_", bs0, t0 == 1 ? cs : nullptr, t0 == 1 ? cdim : 0);
-            // K1: operator A11 (PETSc applies the Schur operator matrix-free for Krylov K1; with preonly only the PC matters),
-            // preconditioner built from the assembled selfp matrix
-            sch->k1 = make_inner(h, sch->S.get(), "preonly", sub_pc, "fp_fieldsplit_1_", bs1, t1 == 1 ? cs : nullptr, t1 == 1 ? cdim : 0);
-            sch->t0.alloc((size_t)sch->n0); sch->t1.alloc((size_t)sch->n1); sch->u0.alloc((size_t)sch->n0);
-            if (sprec == "cc") {
-                // Chebyshev(4) on the pressure mass matrix P_pp (scale-equivariant: the factor is applied to the result)
-                sch->kv = make_inner(h, sch->A11.get(), "preonly", "chebyshev", "fp_fieldsplit_1_visc_", 1, nullptr, 0);
-                sch->tv.alloc((size_t)sch->n1);
+            if (sch->type != FS_SCHUR) {
+                // PETSc's defaults for the sub-solvers: preonly + ILU(0), block Jacobi + ILU(0) on a row-partitioned block
+                const char* sub_pc = c.nranks > 1 ? "bjacobi" : "ilu";
+                const int bs0 = t0 == 1 ? bs_v : 1, bs1 = t1 == 1 ? bs_v : 1;
+                sch->k0 = make_inner(h, sch->A00.get(), "preonly", sub_pc, "fp_fieldsplit_0_", bs0, t0 == 1 ? cs : nullptr, t0 == 1 ? cdim : 0);
+                sch->k1 = make_inner(h, sch->A11.get(), "preonly", sub_pc, "fp_fieldsplit_1_", bs1, t1 == 1 ? cs : nullptr, t1 == 1 ? cdim : 0);
+                sch->t1.alloc((size_t)sch->n1);
+            } else {
+                // selfp: S = A11 - A10 diag(A00)^-1 A01
+                // cc (extension): the diagonal is the lumped mass + drag part of the velocity block, mass_scale * |diag(A_fs)| of
+                // the SYSTEM matrix (A_fs = -(phi^2 / (k_f dt)) M_v with the rows of fluid Dirichlet dofs zeroed, which then get 1),
+                // and the viscous limit visc_scale * P_pp is added in the application (PCSchur::solve1); oracle: SchurLowerCC
+                const std::string sprec = c.opt("-fp_pc_fieldsplit_schur_precondition", "selfp");
+                PORO_REQUIRE(sprec == "selfp" || sprec == "cc", "-fp_pc_fieldsplit_schur_precondition must be selfp or cc");
+                DBuf<double> d_mass;
+                if (sprec == "cc") {
+                    PORO_REQUIRE(!sch->p_first && pc_type == "diagonal", "schur_precondition cc needs pc type 'diagonal' and -fp_pc_fieldsplit_order fp");
+                    PORO_REQUIRE(A != nullptr && c.has_opt("-fp_pc_fieldsplit_schur_cc_mass_scale") && c.has_opt("-fp_pc_fieldsplit_schur_cc_visc_scale"),
+                                 "schur_precondition cc needs A and the -fp_pc_fieldsplit_schur_cc_mass_scale / _visc_scale options (lib/Preconditioner.py sets them)");
+                    PORO_REQUIRE(ns == nf, "schur_precondition cc expects the displacement and velocity fields on the same nodes");
+                    const double ms = c.opt_d("-fp_pc_fieldsplit_schur_cc_mass_scale", 0.0);
+                    sch->visc_scale = c.opt_d("-fp_pc_fieldsplit_schur_cc_visc_scale", 0.0);
+                    PORO_REQUIRE(ms > 0.0 && sch->visc_scale > 0.0, "schur_precondition cc: the two scales must be positive");
+                    Csr Aperm;
+                    const Csr* Ap = &A->raw;
+                    if (!fl.identity) { permute_matrix(h, A->raw, Aperm); Ap = &Aperm; }
+                    auto Afs = extract_block(h, *Ap, of, of + nf, {0});
+                    d_mass.alloc((size_t)nf);
+                    csr_diag(c, Afs->M, d_mass.p);
+                    vec_abs_scale(c, d_mass.p, ms, nf);
+                    PORO_CUDA(cudaStreamSynchronize(c.stream));
+                }
+                DistPlan* plan0 = nullptr;
+                DistPlan* plan1 = nullptr;
+                if (c.nranks > 1 && c.opt_i("-poro_amg_distributed", 1)) { plan0 = sch->A00->plan_for_amg(); plan1 = sch->A11->plan_for_amg(); }
+                if (plan0 && plan1) {
+                    // row-partitioned: exact complement of the owned rows -- the A01 rows and the diagonal of the ghost dofs of split 0
+                    // arrive by one sparse-row and one vector exchange; S gets its own (wider) halo plan
+                    sch->S = std::make_unique<MatOp>();
+                    sch->S->ctx = &c;
+                    sch->S->dplan = std::make_unique<DistPlan>();
+                    dist_selfp_schur(c, *plan0, *plan1, sch->A00->mat(), sch->A01->mat(), sch->A10->mat(), sch->A11->mat(), sch->S->M,
+                                     *sch->S->dplan, d_mass.p);
+                    sch->S->n_owned_cols = sch->n1;
+                } else
+                // single rank (or -poro_amg_distributed 0): from the local (owned) parts
+                {
+                    Csr a00, a01, a10, a11;
+                    local_square(c, *sch->A00, a00);
+                    auto owned_cols = [&](const MatOp& m, int ncols_owned, Csr& o) {
+                        if (m.M.ncols == ncols_owned) { csr_copy(c, m.M, o); PORO_CUDA(cudaStreamSynchronize(c.stream)); return; }
+                        std::vector<int> rmap((size_t)m.M.nrows), cmap((size_t)m.M.ncols, -1);
+                        for (int i = 0; i < m.M.nrows; ++i) rmap[i] = i;
+                        for (int i = 0; i < ncols_owned; ++i) cmap[i] = i;
+                        DBuf<int> d_r(rmap.size()), d_c(cmap.size());
+                        PORO_CUDA(cudaMemcpy(d_r.p, rmap.data(), rmap.size() * 4, cudaMemcpyHostToDevice));
+                        PORO_CUDA(cudaMemcpy(d_c.p, cmap.data(), cmap.size() * 4, cudaMemcpyHostToDevice));
+                        csr_extract(c, m.M, d_r.p, d_c.p, m.M.nrows, ncols_owned, o);
+                    };
+                    owned_cols(*sch->A01, (int)sch->n1, a01);
+                    owned_cols(*sch->A10, (int)sch->n0, a10);
+                    owned_cols(*sch->A11, (int)sch->n1, a11);
+                    DBuf<double> dinv((size_t)sch->n0);
+                    if (d_mass.p) PORO_CUDA(cudaMemcpy(dinv.p, d_mass.p, (size_t)sch->n0 * 8, cudaMemcpyDeviceToDevice));
+                    else csr_diag(c, a00, dinv.p);
+                    std::vector<double> hd((size_t)sch->n0);
+                    PORO_CUDA(cudaMemcpy(hd.data(), dinv.p, hd.size() * 8, cudaMemcpyDeviceToHost));
+                    for (auto& v : hd) v = v != 0.0 ? 1.0 / v : 1.0;
+                    PORO_CUDA(cudaMemcpy(dinv.p, hd.data(), hd.size() * 8, cudaMemcpyHostToDevice));
+                    csr_scale_cols(c, a10, dinv.p);                      // A10 diag(A00)^-1
+                    Csr prod;
+                    csr_spgemm(c, a10, a01, prod);
+                    sch->S = std::make_unique<MatOp>();
+                    sch->S->ctx = &c;
+                    csr_add_scaled(c, a11, prod, -1.0, nullptr, sch->S->M);
+                }
+                const int bs0 = t0 == 1 ? bs_v : 1, bs1 = t1 == 1 ? bs_v : 1;
+                const char* sub_pc = fp_exact_big ? "lu" : "amg";
+                sch->k0 = make_inner(h, sch->A00.get(), "preonly", sub_pc, "fp_fieldsplit_0_", bs0, t0 == 1 ? cs : nullptr, t0 == 1 ? cdim : 0);
+                // K1: operator A11 (PETSc applies the Schur operator matrix-free for Krylov K1; with preonly only the PC matters),
+                // preconditioner built from the assembled selfp matrix
+                sch->k1 = make_inner(h, sch->S.get(), "preonly", sub_pc, "fp_fieldsplit_1_", bs1, t1 == 1 ? cs : nullptr, t1 == 1 ? cdim : 0);
+                sch->t0.alloc((size_t)sch->n0); sch->t1.alloc((size_t)sch->n1); sch->u0.alloc((size_t)sch->n0);
+                if (sprec == "cc") {
+                    // Chebyshev(4) on the pressure mass matrix P_pp (scale-equivariant: the factor is applied to the result)
+                    sch->kv = make_inner(h, sch->A11.get(), "preonly", "chebyshev", "fp_fieldsplit_1_visc_", 1, nullptr, 0);
+                    sch->tv.alloc((size_t)sch->n1);
+                }
             }
             cc.schur = sch.get();
             k->owned_pc = std::move(sch);
@@ -1141,6 +1157,20 @@ int poro_pc_factor_info(poro_pc* pc, const char* name, int64_t* out, int n) {
     const int64_t v[] = {f->n, f->nnz_l, f->nnz_u, f->amalg_zeros, f->nsuper, f->nlevels, f->max_front, f->npert,
                          f->device_bytes, (int64_t)f->flops, (int64_t)std::llround(f->factor_ms * 1e3), f->apply_bytes};
     for (int i = 0; i < n; ++i) out[i] = i < (int)(sizeof v / sizeof v[0]) ? v[i] : 0;
+    API_END
+}
+
+int poro_pc_ilu_info(poro_pc* pc, const char* name, double* out, int n) {
+    API_BEGIN
+    const std::string nm = name ? name : "";
+    KSP* k = find_ksp(pc, nm);
+    if (!k) throw Error("no such inner solver: " + nm);
+    const PCIlu* f = dynamic_cast<const PCIlu*>(k->pc);
+    if (!f) throw Error("inner solver '" + nm + "' is not an incomplete factorisation (its inner PC is " + k->pc->kind() +
+                        "; select it with -<prefix>pc_type ilu or bjacobi)");
+    const double v[] = {(double)f->n, (double)f->L.nnz, (double)f->U.nnz, (double)f->lptr.size() - 1, (double)f->uptr.size() - 1,
+                        f->min_pivot, (double)f->device_bytes, (double)f->apply_bytes};
+    for (int i = 0; i < n; ++i) out[i] = i < (int)(sizeof v / sizeof v[0]) ? v[i] : 0.0;
     API_END
 }
 

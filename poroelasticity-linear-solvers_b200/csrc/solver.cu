@@ -6,10 +6,11 @@
 //                      CGS2), Givens recurrence on the host from (j+2) scalars per step.
 //   KSP::solve_cg      KSPSolve_CG for the inner s_/f_/p_/fp_fieldsplit_0_ solves
 //                      (petsc-options-inexact:12-15,28-31,44-47,82-87).
-//   PCSchur            PCFIELDSPLIT schur (lib/Preconditioner.py:102-118).
+//   PCSchur            PCFIELDSPLIT schur (lib/Preconditioner.py:102-118), additive and multiplicative.
 //   PCBlockCC::apply   PreconditionerCC.apply, 2-way and 3-way (lib/Preconditioner.py:141-250).
 //   AAR::solve         AAR.solve (lib/AAR.py:46-128) including its quirks.
 //   Anderson           AndersonAcceleration.get_next_vector (lib/AndersonAcceleration.py:19-78).
+#include "ilu.cuh"
 #include "solver.cuh"
 #include <algorithm>
 #include <chrono>
@@ -140,6 +141,19 @@ std::unique_ptr<PC> make_pc(Ctx& c, const std::string& pc_type, const Csr& A, in
                             int coord_dim, const std::string& prefix, DistPlan* plan) {
     if (pc_type == "none") return std::make_unique<PCNone>(&c, A.nrows);
     if (pc_type == "jacobi") return std::make_unique<PCJacobi>(&c, A);
+    if (pc_type == "ilu") {
+        if (c.nranks > 1)
+            throw Error("-" + prefix + "pc_type ilu: the block is row-partitioned over " + std::to_string(c.nranks) + " ranks and ILU(0) "
+                        "factors a block on one GPU (PETSc refuses ILU on a parallel MPIAIJ matrix too); -" + prefix + "pc_type bjacobi "
+                        "runs ILU(0) on each rank's owned diagonal block");
+        return std::make_unique<PCIlu>(&c, A, prefix, prefix, false);
+    }
+    if (pc_type == "bjacobi") {       // A is this rank's owned diagonal block (make_inner): no communication
+        const std::string sub = c.opt("-" + prefix + "sub_pc_type", "ilu"), sub_ksp = c.opt("-" + prefix + "sub_ksp_type", "preonly");
+        if (sub != "ilu") throw Error("-" + prefix + "sub_pc_type " + sub + ": block Jacobi supports the sub-PC ilu only");
+        if (sub_ksp != "preonly") throw Error("-" + prefix + "sub_ksp_type " + sub_ksp + ": block Jacobi supports the sub-KSP preonly only");
+        return std::make_unique<PCIlu>(&c, A, prefix, prefix + "sub_", true);
+    }
     bool want_lu = pc_type == "lu" || pc_type == "cholesky";
     if (!plan && use_sparse_lu(c, pc_type, prefix, A.nrows)) return std::make_unique<PCSparseLU>(&c, A, prefix);
     if (want_lu && !plan && A.nrows <=c.opt_i("-poro_dense_lu_limit", 8192)) return std::make_unique<PCDense>(&c, A);
@@ -608,7 +622,10 @@ void PCSchur::apply(const double* x, double* y) {
     Ctx& c = *ctx;
     const double* x0 = x + off0; const double* x1 = x + off1;
     double* y0 = y + off0; double* y1 = y + off1;
-    if (fact == 0) {                       // lower: y0 = K0 x0 ; y1 = K1 (x1 - A10 y0)
+    if (type == FS_ADDITIVE) {             // y0 = K0 x0 ; y1 = K1 x1
+        { ProfScope ps(c, 3); k0->solve(x0, y0); }
+        { ProfScope ps(c, 4); k1->solve(x1, y1); }
+    } else if (fact == 0 || type == FS_MULTIPLICATIVE) {   // lower / multiplicative: y0 = K0 x0 ; y1 = K1 (x1 - A10 y0)
         { ProfScope ps(c, 3); k0->solve(x0, y0); }
         { ProfScope ps(c, 6); A10->apply(y0, t1.p, SPMV_SUB, x1); }
         { ProfScope ps(c, 4); solve1(t1.p, y1); }

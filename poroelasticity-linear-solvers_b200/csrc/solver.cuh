@@ -173,11 +173,14 @@ struct KSP {
     int fields_test(const double* b, const double* xcur, int it);
 };
 
-// PCFIELDSPLIT(schur) on the fp block (lib/Preconditioner.py:102-118, petsc-options-inexact:78-80)
+// PCFIELDSPLIT on the fp block: schur (lib/Preconditioner.py:102-118, petsc-options-inexact:78-80), or PETSc's additive /
+// multiplicative with K1 built on A11 (no S): additive y0 = K0 x0, y1 = K1 x1; multiplicative y1 = K1 (x1 - A10 y0)
+enum FieldsplitType { FS_SCHUR = 0, FS_ADDITIVE = 1, FS_MULTIPLICATIVE = 2 };
 struct PCSchur : PC {
     Ctx* ctx = nullptr;
     bool p_first = true;            // reference order: split 0 = pressure, split 1 = fluid velocity
-    int fact = 0;                   // 0 lower, 1 upper, 2 full, 3 diag
+    int type = FS_SCHUR;
+    int fact = 0;                   // 0 lower, 1 upper, 2 full, 3 diag (schur only)
     int64_t n0 = 0, n1 = 0, off0 = 0, off1 = 0;   // offsets inside the fp vector [f | p]
     std::unique_ptr<MatOp> A00, A01, A10, A11, S;
     std::unique_ptr<KSP> k0, k1;

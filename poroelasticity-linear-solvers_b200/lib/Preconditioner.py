@@ -136,6 +136,15 @@ class PreconditionerCC(object):
         _capi.check(self.ctx.lib.poro_pc_factor_info(self.h, name.encode(), out, len(out)))
         return dict(zip(self.FACTOR_INFO_KEYS, (int(v) for v in out)))
 
+    ILU_INFO_KEYS = ("rows", "nnz_l", "nnz_u", "lower_levels", "upper_levels", "min_pivot", "device_bytes", "apply_bytes")
+
+    def ilu_info(self, name):
+        """ILU(0) of an inner PC ("s","f","p","fp","diff","fp0","fp1"; -<prefix>pc_type ilu or bjacobi) as a dict (keys:
+        ILU_INFO_KEYS, see poro_pc_ilu_info in include/poro.h); raises for an inner PC that is not ILU / bjacobi."""
+        out = (C.c_double * len(self.ILU_INFO_KEYS))()
+        _capi.check(self.ctx.lib.poro_pc_ilu_info(self.h, name.encode(), out, len(out)))
+        return {k: (float(v) if k == "min_pivot" else int(v)) for k, v in zip(self.ILU_INFO_KEYS, out)}
+
     def mg_info(self, name):
         """Geometric multigrid of an inner PC (`-<prefix>pc_type mg`): ([(N, rows, format) per geometric level, finest
         first], number of algebraic levels below); raises for an inner PC that is not `mg`."""
