@@ -13,6 +13,16 @@ namespace poro {
 
 struct Epilogue;
 
+// shared-memory layout of the column region one table reaches from a brick (stencil.cu, brick path).  Axis 0 of a P2
+// column lattice is split by parity (even columns, then odd ones), so that the lanes of a warp -- rows two lattice steps
+// apart -- read consecutive doubles; every component has its own plane of `cs` doubles.
+struct BrickGeom {
+    int lo[3][2], hi[3][2];   // per axis and row parity (1 = odd): reach of the interior classes, relative to the base column
+    int e[3];                 // staged extent per axis in column nodes (the largest over the bricks)
+    int H, W0;                // axis 0: half row of a parity-split row (kc == 2, else 0), row width in doubles
+    int cs;                   // doubles per component plane: W0 * e[1] * e[2]
+};
+
 // everything one generated matrix was built from.  A whole-lattice matrix (one rank, no ghosts) is applied from it; a
 // row-partitioned slab (`slab`) keeps it for the geometry of its geometric transfers (mg.cuh) and stays assembled.
 struct StencilData {
@@ -36,6 +46,15 @@ struct StencilData {
     // warp has the same class, so table reads are broadcasts and no warp diverges on the entry count
     DBuf<int2> wdesc[2];
     int nwarps[2] = {0};
+    // brick path of the 3-D P2 row fields (-poro_stencil_brick, default on): the interior rows, odd or even-interior on
+    // every axis, are applied by CTAs that own a box of row positions and stage the column region the box reaches in
+    // shared memory; the boundary classes run the warps of `wbnd`.  nb / bext: boxes per axis and their extent.
+    int brick = 0;
+    int nb[3] = {0, 0, 0}, bext[3] = {0, 0, 0};
+    BrickGeom bg[9];
+    DBuf<int32_t> soff[9];           // per entry of an interior class: its offset inside the staged region
+    DBuf<int2> wbnd;
+    int nwbnd = 0;
     // next geometric level (poro_mat_set_coarse): the same matrix generated at N / 2, shared with its handle; its own
     // descriptor may link further down (mg.cuh)
     std::shared_ptr<const Csr> coarse;
